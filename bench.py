@@ -16,6 +16,7 @@ batch), c2_streaming (one frame per call, the way slam_node drives the API: ms/f
 at N > 1 the database is sharded over the ranks and the number is ms per detect() across the job).
 --impl reference times the CPU oracle (the reference's algorithm restated: its sources build here only over an Eigen
 stand-in) on all host cores over a bounded sample of the same pairs, same per-pair work.
+--dump-outputs DIR writes the results of the last timed step as DIR/<name>.npy (see dump_outputs).
 """
 import argparse
 import json
@@ -379,6 +380,33 @@ def bind_to_gpu_numa_node(torch, device):
         return {"error": repr(ex)}
 
 
+DUMP_BYTES = 60_000_000   # the files' payload of the whole job: under 64 MB with their headers
+
+
+def dump_outputs(out_dir, ids, recs, rank=0, world=1):
+    """--dump-outputs: what sb_register_batch_dev returned for this rank's pairs in the last timed step, one float64 .npy
+    per result field, rows in generation order (`pair_id` names the pair of each row).  error_history holds the pairs'
+    histories one after the other, history_len[i] values for pair i, so every value written is one the caller received.
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file.  4096 pairs take
+    under 1 MB.  With N ranks each writes its own files (suffix _rank<r>) within DUMP_BYTES / N; above that, a fixed,
+    seeded sample of its pairs."""
+    rec = np.concatenate([r.rec for r in recs])
+    row_bytes = 8 * (1 + 16 + 5 + rec["error_history"].shape[1])   # a pair's fields with a full-length history
+    keep = np.arange(len(rec))
+    cap = DUMP_BYTES // world
+    if len(rec) * row_bytes > cap:
+        keep = np.sort(np.random.default_rng(rank).choice(len(rec), cap // row_bytes, replace=False))
+    rec, hl = rec[keep], rec["history_len"][keep]
+    out = {"pair_id": np.asarray(ids)[keep], "transformation": rec["transformation"].reshape(-1, 4, 4),
+           "final_error": rec["final_error"], "num_iterations": rec["num_iterations"], "converged": rec["converged"],
+           "status": rec["status"], "history_len": hl,
+           "error_history": rec["error_history"][np.arange(rec["error_history"].shape[1]) < hl[:, None]]}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -392,7 +420,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-sub", action="store_true", help="skip the C2 / C3 / C4 sub-results")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
+    sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree, which may be read-only
     if args.impl == "reference":
         return run_reference(args)
 
@@ -499,6 +533,8 @@ def main():
         launches = eng.launch_count - l0
         ms = e0.elapsed_time(e1) / args.steps
         eng.set_profiling(False)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ids, recs, rank, world_size)
         mine = records(recs)
         if gathered is not None:  # the exchange really delivered every rank's records: all 4096 pair ids, once each
             allrec = gathered.cpu().numpy()

@@ -22,19 +22,21 @@ g++ -std=c++17 -O2 -Wall -I$ROOT/include -I/usr/local/cuda/include gather_test.c
 echo "built tests/cpp/gather_test"
 
 # The node's include order and call sites against the mirror, compile-only, in both branches of dense.hpp.
-REF=${SLAM_REFERENCE:-/root/reference}/slam_viz
+# REFERENCE_ROOT: the original project's checkout, where there is one (its include directory goes last)
+REF=${REFERENCE_ROOT:+$REFERENCE_ROOT/slam_viz}
+REF_INC=${REF:+-I$REF/include}
 mkdir -p obj
-g++ -std=c++17 -O1 -Wall -c -I$HOST -I$ROOT/include -I$REF/include call_sites_test.cpp -o obj/call_sites_noeigen.o
-g++ -std=c++17 -O1 -Wall -c -I$ROOT/oracle/eigen_standin -I$HOST -I$ROOT/include -I$REF/include call_sites_test.cpp \
+g++ -std=c++17 -O1 -Wall -c -I$HOST -I$ROOT/include $REF_INC call_sites_test.cpp -o obj/call_sites_noeigen.o
+g++ -std=c++17 -O1 -Wall -c -I$ROOT/oracle/eigen_standin -I$HOST -I$ROOT/include $REF_INC call_sites_test.cpp \
     -o obj/call_sites_eigenapi.o
 echo "compiled tests/cpp/call_sites_test.cpp (no-Eigen and Eigen-API branches)"
 
 # INTEGRATION.md section 1, literally: the reference's UNMODIFIED slam_node.cpp and file_utils.cpp compiled with the
 # mirror directory in front of the reference's include directory (ROS 2 = tests/cpp/ros_stubs, Eigen = the oracle's
 # stand-in, PoseGraph = a GTSAM-free test double), linked against libslam_b200.so.  Needs the reference's sources:
-# where they are absent (the GPU box) the prebuilt binary that travelled with the tree is used.
-if [ -f "$REF/src/ros/slam_node.cpp" ]; then
-    INC="-Iros_stubs -I$ROOT/oracle/eigen_standin -I$HOST -I$ROOT/include -I$REF/include"
+# where they are absent the binary is not built and the tests that run it skip.
+if [ -n "$REF" ] && [ -f "$REF/src/ros/slam_node.cpp" ]; then
+    INC="-Iros_stubs -I$ROOT/oracle/eigen_standin -I$HOST -I$ROOT/include $REF_INC"
     g++ -std=c++17 -O2 -c $INC "$REF/src/ros/slam_node.cpp" -o obj/slam_node.o
     g++ -std=c++17 -O2 -c $INC "$REF/src/core/file_utils.cpp" -o obj/file_utils.o
     g++ -std=c++17 -O2 -Wall -c $INC pose_graph_double.cpp -o obj/pose_graph_double.o
@@ -42,5 +44,5 @@ if [ -f "$REF/src/ros/slam_node.cpp" ]; then
         -L$ROOT/lidar-slam-from-scratch_b200 -lslam_b200 -Wl,-rpath,'$ORIGIN/../../lidar-slam-from-scratch_b200'
     echo "built tests/cpp/slam_node_dropin from $REF (unmodified slam_node.cpp + file_utils.cpp over the mirror headers)"
 else
-    echo "reference sources not found at $REF: keeping the prebuilt tests/cpp/slam_node_dropin"
+    echo "REFERENCE_ROOT does not name the original project's checkout: tests/cpp/slam_node_dropin not built"
 fi

@@ -1,8 +1,8 @@
 """Test-side loader for oracle/_ref/libslam_ref.so: the reference's own sources compiled against the Eigen stand-in
 (oracle/build_ref.sh, oracle/ref_harness.cpp).  TEST INFRASTRUCTURE ONLY.
 
-The library can only be BUILT where /root/reference exists (the development container); the built file travels with
-the snapshot, so `available()` is true on the GPU box too.  Tests that need it skip when it is absent.
+The library can only be BUILT from a checkout of the original project (REFERENCE_ROOT names it; its sources are not
+part of this repository).  Tests that need it skip when it is absent.
 """
 import ctypes as C
 import os
@@ -26,9 +26,10 @@ def _f64(a):
 
 
 def build():
-    """(Re)build when the reference tree is present and the harness or the stand-in is newer than the library."""
-    ref = os.path.join(os.environ.get("REFERENCE_ROOT", "/root/reference"), "slam_viz", "include")
-    if not os.path.isdir(ref):
+    """(Re)build when REFERENCE_ROOT names the original project's checkout and the harness or the stand-in is newer
+    than the library."""
+    root = os.environ.get("REFERENCE_ROOT")
+    if not root or not os.path.isdir(os.path.join(root, "slam_viz", "include")):
         return
     srcs = [os.path.join(ROOT, "oracle", "ref_harness.cpp"), os.path.join(ROOT, "oracle", "build_ref.sh"),
             os.path.join(ROOT, "oracle", "eigen_standin", "Eigen", "Dense")]

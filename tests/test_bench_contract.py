@@ -6,6 +6,7 @@ import glob
 import json
 import os
 import re
+import sys
 
 import pytest
 
@@ -59,3 +60,68 @@ def test_bench_line_has_the_contract_keys(name, d):
         assert {"bound", "achieved", "peak", "unit", "frac", "traffic"} <= set(r) and r["bound"] in ("hbm", "tensor")
         assert abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
         assert d["cpu_baseline"]["cores"] >= 1
+
+
+def test_dump_outputs_files(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float64 .npy per result field, only values the caller received (finite: nothing from
+    past a pair's history length), rows of all files aligned, and above the size cap the same seeded sample of pairs on
+    every run, the cap shared by the ranks of the job."""
+    import numpy as np
+    import slam_b200
+    monkeypatch.syspath_prepend(ROOT)
+    import bench
+
+    def batch(n, seed):
+        rng = np.random.default_rng(seed)
+        r = np.zeros(n, dtype=slam_b200.ICP_DTYPE)
+        r["transformation"] = rng.normal(size=(n, 16))
+        r["final_error"] = rng.uniform(size=n)
+        r["converged"] = rng.integers(0, 2, n)
+        r["status"] = rng.integers(0, 7, n)
+        r["history_len"] = rng.integers(1, 10, n)
+        r["num_iterations"] = r["history_len"] + 100
+        h = rng.uniform(size=r["error_history"].shape)
+        h[np.arange(h.shape[1]) >= r["history_len"][:, None]] = np.nan     # slots past the history must not be written
+        r["error_history"] = h
+        return slam_b200.ICPResultBatch(r)
+
+    recs = [batch(5, 0), batch(3, 1)]
+    ids = np.arange(8) * 64 + 5
+    fields = ("pair_id", "transformation", "final_error", "num_iterations", "converged", "status", "history_len",
+              "error_history")
+
+    def load(d):
+        return {f: np.load(tmp_path / d / (f + ".npy")) for f in fields}
+
+    def rows_match(got, want_ids):
+        """every row k of every file is the result of pair got["pair_id"][k]"""
+        want = {int(i): r for i, r in zip(ids, (x for b in recs for x in b))}
+        hist = np.split(got["error_history"], np.cumsum(got["history_len"].astype(np.int64))[:-1])
+        assert np.array_equal(got["pair_id"], want_ids) and len(hist) == len(want_ids)
+        for k, i in enumerate(want_ids):
+            w = want[int(i)]
+            assert np.array_equal(got["transformation"][k], w.transformation) and got["final_error"][k] == w.final_error
+            assert (got["num_iterations"][k], got["converged"][k], got["status"][k]) == (w.num_iterations, w.converged,
+                                                                                         w.status)
+            assert got["history_len"][k] == len(w.error_history) and np.array_equal(hist[k], w.error_history)
+
+    bench.dump_outputs(str(tmp_path / "all"), ids, recs)
+    assert sorted(os.listdir(tmp_path / "all")) == sorted(f + ".npy" for f in fields)
+    got = load("all")
+    for f, a in got.items():
+        assert a.dtype == np.float64 and np.all(np.isfinite(a)), f
+    rows_match(got, ids)
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 151 * 8)      # room for three of the eight pairs
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), ids, recs)
+    s1 = load("s1")
+    assert len(s1["pair_id"]) == 3 and np.array_equal(s1["pair_id"], load("s2")["pair_id"])
+    assert sum(a.nbytes for a in s1.values()) <= bench.DUMP_BYTES
+    rows_match(s1, s1["pair_id"])
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * 151 * 8)      # two ranks: two pairs each
+    for r in (0, 1):
+        bench.dump_outputs(str(tmp_path / "ranks"), ids, recs, rank=r, world=2)
+    assert sorted(os.listdir(tmp_path / "ranks")) == sorted(f + s + ".npy" for f in fields for s in ("_rank0", "_rank1"))
+    assert sum(np.load(tmp_path / "ranks" / f).nbytes for f in os.listdir(tmp_path / "ranks")) <= bench.DUMP_BYTES

@@ -7,7 +7,10 @@ mirror's no-Eigen branch (tests/cpp/call_sites_test.cpp).  ROS 2 is tests/cpp/ro
 stand-in, slam::PoseGraph is a GTSAM-free test double (tests/cpp/pose_graph_double.cpp).
 
 GPU: that binary runs the node's own process_frame loop (slam_node.cpp:95-175) over synthetic PLY frames on the
-engine, and what it hands to its pose graph (SURVEY.md 8f N4) equals the batch path's sb_odometry_factors."""
+engine, and what it hands to its pose graph (SURVEY.md 8f N4) equals the batch path's sb_odometry_factors.
+
+Both need the original project's sources, which are not part of this repository: REFERENCE_ROOT names a checkout of it,
+and without one these tests skip."""
 import json
 import os
 import subprocess
@@ -20,7 +23,12 @@ import oracle_lib
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CPP = os.path.join(ROOT, "tests", "cpp")
 EXE = os.path.join(CPP, "slam_node_dropin")
-REF = "/root/reference/slam_viz"
+# the original project's checkout (its slam_viz/ directory below it): REFERENCE_ROOT, unset where it is absent
+REF = os.path.join(os.environ["REFERENCE_ROOT"], "slam_viz") if os.environ.get("REFERENCE_ROOT") else None
+
+
+HAVE_REF = REF is not None and os.path.exists(os.path.join(REF, "src", "ros", "slam_node.cpp"))
+NEEDS_REF = "needs the original project's sources: REFERENCE_ROOT names its checkout"
 
 
 def build():
@@ -30,8 +38,15 @@ def build():
     subprocess.check_call(["sh", os.path.join(CPP, "build.sh")])
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "src", "ros", "slam_node.cpp")),
-                    reason="needs the reference's sources (/root/reference)")
+def node_binary():
+    """tests/cpp/slam_node_dropin, built here from the original project's sources; skips the test without them."""
+    if not HAVE_REF:
+        pytest.skip(NEEDS_REF)
+    build()
+    return EXE
+
+
+@pytest.mark.skipif(not HAVE_REF, reason=NEEDS_REF)
 def test_reference_node_compiles_and_links_against_the_mirror():
     build()  # raises if slam_node.cpp / file_utils.cpp / call_sites_test.cpp do not compile or the link fails
     assert os.path.exists(EXE)
@@ -48,11 +63,10 @@ def test_reference_node_compiles_and_links_against_the_mirror():
 
 
 def test_node_binary_refuses_to_run_without_a_gpu(tmp_path):
-    if not os.path.exists(EXE):
-        pytest.skip("tests/cpp/slam_node_dropin not built")
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present: covered by the gpu test")
+    node_binary()
     write_ply(tmp_path / "000000.ply", np.zeros((8, 3), np.float32))
     env = dict(os.environ, SLAM_PARAM_data_dir=str(tmp_path), SLAM_STUB_VERBOSE="1")
     p = subprocess.run([EXE], capture_output=True, text=True, env=env)
@@ -71,8 +85,7 @@ def write_ply(path, xyz32):
 
 @pytest.mark.gpu
 def test_reference_node_runs_on_the_engine_and_hands_off_the_same_factors(tmp_path, synth, engine):
-    if not os.path.exists(EXE):
-        pytest.skip("tests/cpp/slam_node_dropin not built (needs /root/reference at build time)")
+    node_binary()
     scene = synth.scene(5, n_boxes=400)
     s = oracle_lib.small_sensor(32, 600)
     n_frames = 7

@@ -1,5 +1,5 @@
-"""The CPU oracle against the REFERENCE'S OWN SOURCES (oracle/_ref/libslam_ref.so: /root/reference/slam_viz compiled
-unmodified against oracle/eigen_standin, see oracle/build_ref.sh).
+"""The CPU oracle against the REFERENCE'S OWN SOURCES (oracle/_ref/libslam_ref.so: $REFERENCE_ROOT/slam_viz, a checkout
+of the original project, compiled unmodified against oracle/eigen_standin, see oracle/build_ref.sh).
 
 What this pins: every piece of the reference's control flow on the hot path -- the voxel hash map and its centroid
 order, KD-tree build (nth_element medians) and both searches, the normal orientation rule, the ICP loop with its
@@ -8,7 +8,8 @@ loop-closure candidate filter, sort and sequential acceptance, float32 loaders. 
 floating-point kernels (eigen solver, LDLT, reductions), which the stand-in replaces with plain fp64 loops; the
 tolerances below (1e-9 and tighter) are there for that substitution only.
 
-Skipped when the library is absent (it can be built only where /root/reference exists; the built file travels).
+Skipped when the library is absent: it can be built only from the original project's sources, which are not part of
+this repository.
 """
 import numpy as np
 import pytest
