@@ -219,6 +219,31 @@ int sb_loop_candidates_local(sb_loop* loop, double* dist, int32_t* entry, int32_
 int sb_loop_verify_entries(sb_loop* loop, const int32_t* entry, const double* dist, int32_t n, sb_loop_result* results,
                            int32_t* converged);
 
+/* Loop-closure detection over a whole recorded sequence.  The node calls addFrame and detect() once per keyframe
+ * (slam_node.cpp:159-167, loop_closure.hpp:53-126); detect() for the query entry q reads only entries 0..q-1, so the
+ * detections of many query entries are independent and run here as one many-query search and batched ICP rounds.
+ *
+ * addFrame for n_frames clouds at once: host fp64 rows in CSR form (cloud f is rows [offsets[f], offsets[f+1]),
+ * offsets[0] = 0), frame_idx[n_frames], desc: n_frames*1200 Scan Context descriptors or NULL (computed).  Leaves the
+ * detector in exactly the state n_frames calls of sb_loop_add_frame_desc would (world > 1 included: the owned entries
+ * are kept, and the newest entry as a guest).  One descriptor launch and one synchronise. */
+int sb_loop_add_frames(sb_loop* loop, const double* xyz, const int64_t* offsets, int32_t n_frames,
+                       const int32_t* frame_idx, const double* desc);
+/* Largest k of sb_loop_candidates_batch: the short list selected on the device per query. */
+#define SB_LOOP_SELECT_MAX 32
+/* Stage 1 of detect() for many queries (world == 1).  query_entries: n_queries entry ids, strictly ascending, each
+ * below sb_loop_size.  Query q_i sees the entries e < q_i with frame[q_i] - frame[e] >= frame_gap and distance <
+ * threshold (loop_closure.hpp:75-92): the best min(k, count[i]) of them, ascending by (distance, entry), are at
+ * dist / entry[i*k ...]; count[i] = how many there are.  1 <= k <= SB_LOOP_SELECT_MAX. */
+int sb_loop_candidates_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries, int32_t k,
+                             double* dist, int32_t* entry, int32_t* count);
+/* detect() for many queries (world == 1, same query_entries rules): the result for q_i is what sb_loop_detect returns
+ * right after entry q_i was added (query_frame = frame[q_i]).  results[i*max_candidates ...] holds the count[i]
+ * accepted loops of query i.  The walk down each candidate list never skips a candidate.  The detector is not
+ * modified.  max_candidates <= 0 gives empty results (results may then be NULL). */
+int sb_loop_detect_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries,
+                         sb_loop_result* results, int32_t* count);
+
 /* ---------------------------------------------------------------- after the path: world frame, map -------- */
 /* The data-parallel steps that follow registration in slam_node.cpp (SURVEY.md 8f N2/N3).  poses16: n_clouds
  * row-major 4x4 transforms (Transformation::matrix()), cloud c is rows [offsets[c], offsets[c+1]). */

@@ -1067,7 +1067,8 @@ int sb_loop_verify_entries(sb_loop* loop, const int32_t* entry, const double* di
                            int32_t* converged) {
     if (!loop || n < 0 || (n > 0 && (!entry || !results || !converged))) return SB_ERR_INVALID_ARG;
     Enter g(loop->ctx);
-    return loop_verify(loop, entry, dist, n, results, converged);
+    const std::vector<int> qslots((size_t)n, (int)loop->entry_id.size() - 1);   // the newest entry is the query
+    return loop_verify(loop, qslots.data(), entry, dist, n, results, converged);
 }
 
 int sb_loop_detect(sb_loop* loop, sb_loop_result* results, int32_t capacity, int32_t* count) {
@@ -1099,8 +1100,9 @@ int sb_loop_detect(sb_loop* loop, sb_loop_result* results, int32_t capacity, int
         std::vector<double> dist((size_t)m);
         std::vector<sb_loop_result> res((size_t)m);
         for (int i = 0; i < m; ++i) { ent[i] = cand[b + i].second; dist[i] = cand[b + i].first; }
+        const std::vector<int> qslots((size_t)m, (int)loop->entry_id.size() - 1);
         arena_reset(c);
-        SB_TRY(loop_verify(loop, ent.data(), dist.data(), m, res.data(), conv.data()));
+        SB_TRY(loop_verify(loop, qslots.data(), ent.data(), dist.data(), m, res.data(), conv.data()));
         for (int i = 0; i < m && verified < loop->cfg.max_candidates; ++i) {
             if (conv[i] && res[i].icp_fitness < loop->cfg.icp_fitness_threshold) {  // loop_closure.hpp:112
                 if (*count < capacity) results[*count] = res[i];
@@ -1110,6 +1112,61 @@ int sb_loop_detect(sb_loop* loop, sb_loop_result* results, int32_t capacity, int
         }
     }
     return SB_OK;
+}
+
+int sb_loop_add_frames(sb_loop* loop, const double* xyz, const int64_t* offsets, int32_t n_frames,
+                       const int32_t* frame_idx, const double* desc) {
+    if (!loop || n_frames < 0 || (n_frames > 0 && (!offsets || !frame_idx))) return SB_ERR_INVALID_ARG;
+    Ctx* c = loop->ctx;
+    Enter g(c);
+    if (n_frames == 0) return SB_OK;
+    if (offsets[0] != 0) return fail(c, SB_ERR_INVALID_ARG, "offsets must start at 0");
+    for (int i = 0; i < n_frames; ++i)
+        if (offsets[i + 1] < offsets[i]) return fail(c, SB_ERR_INVALID_ARG, "offsets must be non-decreasing");
+    if (offsets[n_frames] > 0 && !xyz) return fail(c, SB_ERR_INVALID_ARG, "null buffer");
+    return loop_add_many(loop, xyz, reinterpret_cast<const i64*>(offsets), n_frames, frame_idx, desc);
+}
+
+// query entry ids of the batch entry points: world == 1 (entry id = slot), strictly ascending, below size()
+static int check_queries(sb_loop* loop, const int32_t* q, int32_t n) {
+    Ctx* c = loop->ctx;
+    if (loop->world != 1) return fail(c, SB_ERR_INVALID_ARG, "batch loop detection needs world == 1");
+    for (int i = 0; i < n; ++i) {
+        if (q[i] < 0 || q[i] >= loop->n_global)
+            return fail(c, SB_ERR_INVALID_ARG, "query entry %d out of range [0, %d)", q[i], loop->n_global);
+        if (i > 0 && q[i] <= q[i - 1]) return fail(c, SB_ERR_INVALID_ARG, "query entries must be strictly ascending");
+    }
+    return SB_OK;
+}
+
+int sb_loop_candidates_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries, int32_t k, double* dist,
+                             int32_t* entry, int32_t* count) {
+    if (!loop || n_queries < 0 || k < 1 || k > SB_LOOP_SELECT_MAX ||
+        (n_queries > 0 && (!query_entries || !dist || !entry || !count)))
+        return SB_ERR_INVALID_ARG;
+    Enter g(loop->ctx);
+    SB_TRY(check_queries(loop, query_entries, n_queries));
+    std::vector<std::vector<std::pair<double, int>>> cand;
+    std::vector<int> total;
+    SB_TRY(loop_candidates_batch(loop, query_entries, n_queries, cand, total));
+    for (int i = 0; i < n_queries; ++i) {
+        count[i] = total[i];
+        for (int j = 0; j < k && j < (int)cand[i].size(); ++j) {
+            dist[(size_t)i * k + j] = cand[i][j].first;
+            entry[(size_t)i * k + j] = cand[i][j].second;
+        }
+    }
+    return SB_OK;
+}
+
+int sb_loop_detect_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries, sb_loop_result* results,
+                         int32_t* count) {
+    if (!loop || n_queries < 0 || (n_queries > 0 && (!query_entries || !count)) ||
+        (n_queries > 0 && loop->cfg.max_candidates > 0 && !results))
+        return SB_ERR_INVALID_ARG;
+    Enter g(loop->ctx);
+    SB_TRY(check_queries(loop, query_entries, n_queries));
+    return loop_detect_batch(loop, query_entries, n_queries, results, count);
 }
 
 // ---------------------------------------------------------------- after the path: world frame, map

@@ -367,6 +367,12 @@ int sc_compute_dev(Ctx* ctx, const double* d_xyz, const i64* d_off, int n_clouds
 // one query descriptor against n_db descriptors (all column-major 20x60, device)
 int sc_distance_dev(Ctx* ctx, const double* d_query_desc, const double* d_db, int n_db, double* d_out);
 int sc_keys_dev(Ctx* ctx, const double* d_desc, double* d_ring, double* d_sector);
+// sq[e * 60 + s]: the shifted self sum sum_bb(e, s) of k_sc_distance for n descriptors
+int sc_sq_dev(Ctx* ctx, const double* d_desc, int n, double* d_sq);
+// Many queries: dist[r * ld + e] = distance of query slot qslot[r] (ascending) to entry slot e, for the entries
+// e < n_e of every tile that holds a pair with e < qslot[r] and a frame gap >= frame_gap (d_meta: (frame, entry))
+int sc_distance_many_dev(Ctx* ctx, const double* d_desc, const double* d_sq, const int2* d_meta, const int* d_qslot,
+                         int n_q, int n_e, int frame_gap, double* d_dist, i64 ld);
 
 // icp.cu
 int solve_point_to_plane_dev(Ctx* ctx, const double* d_src, const double* d_tgt, const double* d_nrm, i64 n,
@@ -414,7 +420,14 @@ int loop_add(sb_loop* L, const double* xyz, i64 n, int frame_idx, const double* 
 int loop_reserve(sb_loop* L, i64 n_entries, i64 total_rows);
 // limit > 0: at most `limit` (<= SB_LOOP_SELECT_MAX) best candidates, selected on the device; limit <= 0: all of them.
 // *total: number of candidates under the threshold either way.
-#define SB_LOOP_SELECT_MAX 32
-int loop_candidates(sb_loop* L, std::vector<std::pair<double, int>>& cand, int limit, int* total);
-int loop_verify(sb_loop* L, const int* entries, const double* dist, int n, sb_loop_result* results, int* converged);
+// qslot: the query's local slot (entries before it are searched); -1: the newest entry.
+int loop_candidates(sb_loop* L, std::vector<std::pair<double, int>>& cand, int limit, int* total, int qslot = -1);
+// ICP(query cloud of slot qslots[i] -> cloud of entry entries[i]) for every i.
+int loop_verify(sb_loop* L, const int* qslots, const int* entries, const double* dist, int n, sb_loop_result* results,
+                int* converged);
+// Batch entry points (world == 1 for the two queries; query slots strictly ascending).
+int loop_add_many(sb_loop* L, const double* xyz, const i64* offsets, int n_frames, const int* frame_idx, const double* desc);
+int loop_candidates_batch(sb_loop* L, const int* qslots, int n_q, std::vector<std::vector<std::pair<double, int>>>& cand,
+                          std::vector<int>& total);
+int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* results, int* count);
 }  // namespace sb

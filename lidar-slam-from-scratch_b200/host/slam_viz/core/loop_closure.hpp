@@ -1,6 +1,7 @@
 // loop_closure.hpp — mirror of slam_viz/include/slam_viz/core/loop_closure.hpp:14-149.
 // The descriptor database and the cloud copies live in device memory (csrc/loop.cu).
 #pragma once
+#include <algorithm>
 #include <memory>
 #include <vector>
 
@@ -48,15 +49,7 @@ public:
         int32_t count = 0;
         b200::check(sb_loop_detect(loop_.get(), raw.data(), cap, &count), "detect");
         std::vector<LoopClosureResult> out;
-        for (int i = 0; i < count && i < cap; ++i) {
-            LoopClosureResult r;
-            r.query_frame = raw[i].query_frame;
-            r.match_frame = raw[i].match_frame;
-            r.transform = Transformation::from_row_major(raw[i].transform);
-            r.scan_context_distance = raw[i].scan_context_distance;
-            r.icp_fitness = raw[i].icp_fitness;
-            out.push_back(r);
-        }
+        for (int i = 0; i < count && i < cap; ++i) out.push_back(result(raw[i]));
         return out;
     }
 
@@ -66,8 +59,42 @@ public:
     void reserve(size_t frames, size_t total_rows) {
         b200::check(sb_loop_reserve(loop_.get(), (int64_t)frames, (int64_t)total_rows), "reserve");
     }
+    // extension: addFrame for every cloud of a recorded sequence in one call (same state as one addFrame per cloud)
+    void addFrames(const std::vector<PointCloud::Matrix>& clouds, const std::vector<int>& frame_idx) {
+        if (clouds.size() != frame_idx.size()) b200::check(SB_ERR_INVALID_ARG, "addFrames: one frame index per cloud");
+        std::vector<int64_t> off(1, 0);
+        for (const auto& c : clouds) off.push_back(off.back() + (int64_t)c.rows());
+        std::vector<double> xyz((size_t)off.back() * 3);
+        for (size_t f = 0; f < clouds.size(); ++f)
+            std::copy(clouds[f].data(), clouds[f].data() + 3 * clouds[f].rows(), xyz.begin() + 3 * off[f]);
+        std::vector<int32_t> fi(frame_idx.begin(), frame_idx.end());
+        b200::check(sb_loop_add_frames(loop_.get(), xyz.data(), off.data(), (int32_t)clouds.size(), fi.data(), nullptr),
+                    "addFrames");
+    }
+    // extension: detect() as it would have answered right after each listed entry (strictly ascending) was added
+    std::vector<std::vector<LoopClosureResult>> detectBatch(const std::vector<int>& query_entries) {
+        const int cap = config_.max_candidates > 0 ? config_.max_candidates : 0;
+        const size_t n = query_entries.size();
+        std::vector<int32_t> q(query_entries.begin(), query_entries.end()), count(n > 0 ? n : 1, 0);
+        std::vector<sb_loop_result> raw(n * (size_t)cap > 0 ? n * (size_t)cap : 1);
+        b200::check(sb_loop_detect_batch(loop_.get(), q.data(), (int32_t)n, raw.data(), count.data()), "detectBatch");
+        std::vector<std::vector<LoopClosureResult>> out(n);
+        for (size_t i = 0; i < n; ++i)
+            for (int j = 0; j < count[i]; ++j) out[i].push_back(result(raw[i * (size_t)cap + j]));
+        return out;
+    }
 
 private:
+    static LoopClosureResult result(const sb_loop_result& raw) {
+        LoopClosureResult r;
+        r.query_frame = raw.query_frame;
+        r.match_frame = raw.match_frame;
+        r.transform = Transformation::from_row_major(raw.transform);
+        r.scan_context_distance = raw.scan_context_distance;
+        r.icp_fitness = raw.icp_fitness;
+        return r;
+    }
+
     LoopClosureConfig config_;
     std::shared_ptr<sb_loop> loop_;
 };

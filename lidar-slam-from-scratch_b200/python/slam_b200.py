@@ -10,6 +10,7 @@ names and argument meaning to Python callers (tests, bench.py) on top of the C A
     icp_point_to_plane(source, target, cfg)    icp.hpp:157-258
     ScanContext(cloud).distance(other)         scan_context.hpp:24-145
     LoopClosureDetector(cfg).addFrame/detect   loop_closure.hpp:41-149
+    LoopClosureDetector.addFrames/detect_batch the same over a whole recorded sequence (slam_node.cpp:159-167)
 
 There is no CPU implementation here: if the shared library is missing, or no sm_100 device is usable, construction
 fails loudly.
@@ -26,6 +27,7 @@ _LIB_PATH = os.environ.get("SB_LIB_PATH") or os.path.join(os.path.dirname(_HERE)
 SB_SC_SIZE = 1200
 SB_MAX_K = 32
 SB_MAX_ICP_ITERATIONS = 128
+SB_LOOP_SELECT_MAX = 32
 
 STATUS = {0: "SB_OK", 1: "SB_ERR_INVALID_ARG", 2: "SB_ERR_EMPTY", 3: "SB_ERR_CUDA", 4: "SB_ERR_NO_DEVICE",
           5: "SB_ERR_RANGE", 6: "SB_ERR_CAPACITY"}
@@ -122,6 +124,9 @@ SYMBOLS = {
     "sb_loop_detect": (C.c_int, [_P, C.POINTER(LoopResultC), C.c_int32, _I32]),
     "sb_loop_candidates_local": (C.c_int, [_P, _D, _I32, C.c_int32, _I32]),
     "sb_loop_verify_entries": (C.c_int, [_P, _I32, _D, C.c_int32, C.POINTER(LoopResultC), _I32]),
+    "sb_loop_add_frames": (C.c_int, [_P, _D, _I64, C.c_int32, _I32, _D]),
+    "sb_loop_candidates_batch": (C.c_int, [_P, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
+    "sb_loop_detect_batch": (C.c_int, [_P, _I32, C.c_int32, C.POINTER(LoopResultC), _I32]),
     "sb_odometry_poses": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_double, _D, _D]),
     "sb_gather_results": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(ICPResultC), C.c_int32, C.POINTER(ICPResultC)]),
     "sb_gather_candidates": (C.c_int, [_P, _P, C.c_int32, _D, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
@@ -678,3 +683,39 @@ class LoopClosureDetector:
         self.e._check(self.e.lib.sb_loop_verify_entries(self.h, ent.ctypes.data_as(_I32), _dp(d), n, res,
                                                         conv.ctypes.data_as(_I32)))
         return [self._result(res[i]) for i in range(n)], conv[:n].astype(bool)
+
+    def addFrames(self, xyz, offsets, frame_idx, descs=None):
+        """addFrame for every cloud of a CSR batch (cloud f = rows offsets[f]:offsets[f+1]) in one call; descs: optional
+        (n_frames, 1200) Scan Context descriptors.  Same detector state as one addFrame per cloud."""
+        p = _f64(xyz, 3)
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        fi = np.ascontiguousarray(frame_idx, dtype=np.int32)
+        n = off.shape[0] - 1
+        if fi.shape[0] != n:
+            raise ValueError("frame_idx needs one frame per cloud")
+        d = None if descs is None else _f64(descs).reshape(n, SB_SC_SIZE)
+        self.e._check(self.e.lib.sb_loop_add_frames(self.h, _dp(p), off.ctypes.data_as(_I64), n, fi.ctypes.data_as(_I32),
+                                                    _dp(d) if d is not None else None))
+
+    def candidates_batch(self, query_entries, k=SB_LOOP_SELECT_MAX):
+        """Stage 1 of detect() for every listed query entry (strictly ascending): per query the best min(k, count)
+        (distance, entry) pairs as arrays, and the number of candidates under the threshold."""
+        q = np.ascontiguousarray(query_entries, dtype=np.int32)
+        n = q.shape[0]
+        dist = np.empty((max(n, 1), k))
+        ent = np.empty((max(n, 1), k), dtype=np.int32)
+        cnt = np.zeros(max(n, 1), dtype=np.int32)
+        self.e._check(self.e.lib.sb_loop_candidates_batch(self.h, q.ctypes.data_as(_I32), n, int(k), _dp(dist),
+                                                          ent.ctypes.data_as(_I32), cnt.ctypes.data_as(_I32)))
+        return [(dist[i, :min(cnt[i], k)].copy(), ent[i, :min(cnt[i], k)].copy()) for i in range(n)], cnt[:n].copy()
+
+    def detect_batch(self, query_entries):
+        """detect() as it would have answered right after each listed entry (strictly ascending) was added: a list of
+        per-query lists of the dicts detect() returns."""
+        q = np.ascontiguousarray(query_entries, dtype=np.int32)
+        n = q.shape[0]
+        m = max(int(self.cfg.max_candidates), 0)
+        res = (LoopResultC * max(n * m, 1))()
+        cnt = np.zeros(max(n, 1), dtype=np.int32)
+        self.e._check(self.e.lib.sb_loop_detect_batch(self.h, q.ctypes.data_as(_I32), n, res, cnt.ctypes.data_as(_I32)))
+        return [[self._result(res[i * m + j]) for j in range(cnt[i])] for i in range(n)]
