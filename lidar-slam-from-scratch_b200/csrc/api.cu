@@ -347,6 +347,18 @@ static int register_batch_impl(Ctx* ctx, PointSrc src, const void* h_raw, const 
     // grid / index / normals of the next chunk instead of in front of them.  Results do not depend on how the pairs
     // are grouped (every pair's sums are added in its own fixed order).
     bool pipelined = false;   // set on the chunked host path: index_clouds then also starts the ICP of the ready pairs
+    // the pipelined path leaves work on three streams; every return, an error exit included, waits for all of it,
+    // because the next call reuses the arena and the staging buffers as soon as it enters
+    struct Drain {
+        Ctx* c;
+        const bool& on;
+        ~Drain() {
+            if (!on) return;
+            if (c->icp_stream) cudaStreamSynchronize(c->icp_stream);
+            if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+            cudaStreamSynchronize(c->stream);
+        }
+    } drain{ctx, pipelined};
     std::vector<char> launched((size_t)n_pairs, 0);
     std::vector<IcpPending> pending;
     std::vector<std::vector<int>> pending_ids;
@@ -356,6 +368,9 @@ static int register_batch_impl(Ctx* ctx, PointSrc src, const void* h_raw, const 
         for (int p = 0; p < n_pairs; ++p)
             if (!launched[p] && pair_src[p] < c1 && pair_tgt[p] < c1) ids.push_back(p);
         if (ids.empty() || (!last && (int)ids.size() < sub_min)) return SB_OK;
+        // one staging slot per sub-batch (Ctx::ICP_SLOTS): when only the last one is left, the ready pairs wait for the
+        // last chunk and go with its sub-batch
+        if (!last && (int)pending.size() >= Ctx::ICP_SLOTS - 1) return SB_OK;
         std::vector<PairDesc> pairs(ids.size());
         for (size_t i = 0; i < ids.size(); ++i) {
             const int p = ids[i];
@@ -558,6 +573,8 @@ void sb_ctx_destroy(sb_ctx* ctx) {
     if (!ctx) return;
     Ctx* c = &ctx->c;
     cudaSetDevice(c->device);
+    if (c->icp_stream) cudaStreamSynchronize(c->icp_stream);
+    if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     cudaStreamSynchronize(c->stream);
     icp_graph_free(c);
     for (void* p : c->arena.overflow) cudaFree(p);

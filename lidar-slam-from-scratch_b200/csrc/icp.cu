@@ -1082,6 +1082,10 @@ int icp_enqueue(Ctx* ctx, const Forest* f, const std::vector<PairDesc>& pairs_in
         return fail(ctx, SB_ERR_INVALID_ARG, "icp: max_iterations %d outside [0, %d]", cfg->max_iterations,
                     SB_MAX_ICP_ITERATIONS);
     if (f->normals_k <= 0) return fail(ctx, SB_ERR_INVALID_ARG, "icp: forest has no normals");
+    // staging for the results and the pass count: checked before anything is enqueued, so that a batch that cannot be
+    // staged launches nothing
+    if (ctx->icp_res_used + (size_t)n_pairs > ctx->icp_res_cap || ctx->icp_slots_used >= Ctx::ICP_SLOTS)
+        return fail(ctx, SB_ERR_CAPACITY, "icp: result staging full (icp_reserve_results sizes it per call)");
     IcpGraph* G;
     SB_TRY(icp_graph_get(ctx, &G));
     std::vector<PairDesc> pairs(pairs_in);
@@ -1174,8 +1178,6 @@ int icp_enqueue(Ctx* ctx, const Forest* f, const std::vector<PairDesc>& pairs_in
         SB_LAUNCH(ctx, k_icp_solve, G->solve_grid, 256, 0, G->d_job, 1, none, 0);
     }
     // results and the pass count: into pinned host memory, asynchronously
-    if (ctx->icp_res_used + (size_t)n_pairs > ctx->icp_res_cap || ctx->icp_slots_used >= Ctx::ICP_SLOTS)
-        return fail(ctx, SB_ERR_CAPACITY, "icp: result staging full (icp_reserve_results sizes it per call)");
     out->slot = ctx->icp_slots_used++;
     ctx->icp_res_used += (size_t)n_pairs;
     SB_CUDA(ctx, cudaMemcpyAsync(ctx->h_icp_res + out->h_off, d_res, sizeof(sb_icp_result) * n_pairs, cudaMemcpyDeviceToHost,
