@@ -244,6 +244,61 @@ int sb_loop_candidates_batch(sb_loop* loop, const int32_t* query_entries, int32_
 int sb_loop_detect_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries,
                          sb_loop_result* results, int32_t* count);
 
+/* ---------------------------------------------------------------- streaming odometry session --------------- */
+/* SlamNode::process_frame (slam_node.cpp:118-175) one scan per call, with the previous frame kept on the device: its
+ * downsampled cloud, index and normals serve as the next frame's ICP target, so no frame is uploaded or indexed twice.
+ * A session belongs to one context; the optional loop-closure detector must be created on the same context and must
+ * outlive the session.  Per push:
+ *   1. voxel grid (slam_node.cpp:122); fewer than min_points rows: the frame is SKIPPED (slam_node.cpp:125-130): the
+ *      pose is repeated, the previous frame stays the ICP target, nothing is added and detect does not run;
+ *   2. ICP of this frame (source) onto the previous one (target), exactly sb_icp_point_to_plane(current, previous, icp);
+ *   3. pose = previous pose * delta with sb_odometry_poses's rule and arithmetic (the first frame: the initial pose);
+ *   4. the world-frame cloud as PointCloud2 float32 records (sb_transform_clouds_f32) and the Scan Context (sb_sc_compute);
+ *   5. SB_ODOM_ADD_FRAME: the detector is left in the state sb_loop_add_frame(cloud, frame_idx) leaves (world > 1 too);
+ *   6. SB_ODOM_DETECT (world == 1 only): loops = what sb_loop_detect_batch returns for the detector's newest entry.
+ * A call that fails (SB_ERR_INVALID_ARG, SB_ERR_EMPTY, SB_ERR_RANGE, ...) leaves the session and the detector as they
+ * were: the next push behaves as if the failed one had never been made. */
+typedef struct sb_odom sb_odom;
+typedef struct sb_odom_config {
+    double voxel;              /* 0.5   slam_node voxel_size; <= 0: no voxel grid                                     */
+    int32_t min_points;        /* 1000  slam_node.hpp:29: fewer rows after the voxel grid -> the frame is skipped      */
+    int32_t reserved;
+    double max_error;          /* 1.0   slam_node.cpp:139-140: delta = identity if final_error > max_error            */
+    sb_icp_config icp;         /* sb_default_icp_config                                                              */
+    double initial_pose[16];   /* row-major 4x4, identity                                                            */
+} sb_odom_config;
+void sb_default_odom_config(sb_odom_config* cfg);
+/* loop: NULL for no loop closure, else a detector created on ctx */
+int sb_odom_create(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_odom** out);
+void sb_odom_free(sb_odom* odom);
+/* Optional: size every device and pinned buffer for frames of up to max_raw_rows rows, so that no push allocates. */
+int sb_odom_reserve(sb_odom* odom, int64_t max_raw_rows);
+/* Continue the pose chain from pose16 (row-major), e.g. an optimised pose (slam_node.cpp:177-185). */
+int sb_odom_set_pose(sb_odom* odom, const double* pose16);
+/* The pose of the newest registered (or first) frame. */
+int sb_odom_get_pose(const sb_odom* odom, double* pose16);
+
+enum { SB_ODOM_ADD_FRAME = 1, SB_ODOM_DETECT = 2 };          /* per-push flags */
+enum { SB_ODOM_FIRST = 0, SB_ODOM_REGISTERED = 1, SB_ODOM_SKIPPED = 2 };
+typedef struct sb_odom_frame {
+    int32_t frame_idx, state;  /* state: SB_ODOM_FIRST | SB_ODOM_REGISTERED | SB_ODOM_SKIPPED                         */
+    int64_t n_points;          /* rows after the voxel grid                                                          */
+    double pose[16];           /* pose of this frame after the chain step (skipped: the previous pose)                */
+    sb_icp_result icp;         /* state == SB_ODOM_REGISTERED, else zero                                             */
+    int32_t n_loops, pad;      /* accepted loop closures (SB_ODOM_DETECT), counted like sb_loop_detect's *count       */
+} sb_odom_frame;
+/* xyz: n host fp64 rows.  Outputs (NULL: not wanted): out_xyz n_points*3 doubles (downsampled rows, sensor frame; also
+ * for a skipped frame), out_world_f32 n_points*3 floats and out_desc 1200 doubles (not for a skipped frame), loops: the
+ * first min(n_loops, loop_capacity) accepted loop closures (NULL only with loop_capacity == 0).  The output buffers must
+ * hold n rows: n_points is not known before the call. */
+int sb_odom_push(sb_odom* odom, const double* xyz, int64_t n, int32_t frame_idx, int32_t flags, sb_odom_frame* out,
+                 double* out_xyz, float* out_world_f32, double* out_desc, sb_loop_result* loops, int32_t loop_capacity);
+/* The float32 records of a PLY / KITTI file: rows of stride_floats (>= 3) floats, x, y, z first, widened on the device
+ * (as sb_register_batch_f32): the same results as sb_odom_push of the widened rows. */
+int sb_odom_push_f32(sb_odom* odom, const float* xyz, int32_t stride_floats, int64_t n, int32_t frame_idx,
+                     int32_t flags, sb_odom_frame* out, double* out_xyz, float* out_world_f32, double* out_desc,
+                     sb_loop_result* loops, int32_t loop_capacity);
+
 /* ---------------------------------------------------------------- after the path: world frame, map -------- */
 /* The data-parallel steps that follow registration in slam_node.cpp (SURVEY.md 8f N2/N3).  poses16: n_clouds
  * row-major 4x4 transforms (Transformation::matrix()), cloud c is rows [offsets[c], offsets[c+1]). */

@@ -168,18 +168,6 @@ int pinned_reserve(Ctx* ctx, size_t bytes) {
     return SB_OK;
 }
 
-// RAII entry guard: selects the device and resets the arena
-struct Enter {
-    Ctx* c;
-    explicit Enter(Ctx* ctx) : c(ctx) {
-        cudaSetDevice(c->device);
-        arena_reset(c);
-        c->tbuf_used = 0;  // everything the previous call enqueued has completed
-        c->err.clear();
-        c->n_ev = 0;
-    }
-};
-
 static int upload(Ctx* ctx, const void* h, size_t bytes, void** d) {
     SB_TRY(arena_alloc(ctx, bytes, d));
     if (bytes) SB_CUDA(ctx, cudaMemcpyAsync(*d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));

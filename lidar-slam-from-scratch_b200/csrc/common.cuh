@@ -174,6 +174,13 @@ __device__ __forceinline__ float sqrt_upper(double d2) { return __fmul_ru(sqrt_a
 
 __device__ __forceinline__ double shfl_d_xor(double v, int m) { return __shfl_xor_sync(0xffffffffu, v, m); }
 
+// Row a of T * p for a row-major 4x4 T: p * R^T + t with the association of Transformation::apply (types.hpp:110-115).
+// Every world-frame transform of the library (mapping.cu's k_transform, odom.cu's epilogue) goes through this one
+// expression, so their bits cannot drift apart.
+__device__ __forceinline__ double apply_row(const double* T, int a, double x, double y, double z) {
+    return ((x * T[4 * a] + y * T[4 * a + 1]) + z * T[4 * a + 2]) + T[4 * a + 3];
+}
+
 __device__ __forceinline__ unsigned lanemask_lt() {
     unsigned m;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
@@ -286,6 +293,21 @@ struct ForestBatch {    // the arrays of the trees [t0, t0 + n_trees) appended t
     GridSlot* grid = nullptr;
 };
 
+// Caller-owned arrays for ONE batch of trees (odom.cu's frame slots): sized up front by the caller, never allocated or
+// freed by the forest.  forest_append / forest_normals fail with SB_ERR_CAPACITY if the batch does not fit.
+struct TreeStore {
+    TreePoint* pts = nullptr;
+    float4* pts32 = nullptr;
+    float* boxes = nullptr;
+    TreeNormal* normals = nullptr;
+    NbrEntry* nbr = nullptr;
+    GridSlot* grid = nullptr;
+    i64 cap_points = 0, cap_boxes = 0, cap_slots = 0;
+    int cap_k = 0;
+};
+// What the arrays of one tree over n points need: boxes of all levels and seed-grid slots (forest_append's layout).
+void tree_store_need(i64 n, i64* boxes, i64* slots);
+
 struct Forest {
     Ctx* ctx = nullptr;
     int n_trees = 0, cap_trees = 0;
@@ -295,6 +317,7 @@ struct Forest {
     std::vector<TreeDesc> h_trees;   // host mirror (the seed-grid fields glo/gext/ginv are device-only)
     int normals_k = 0;      // 0: no normals yet
     bool in_arena = false;  // arrays live in the context arena (valid until the next C-ABI call), not cudaMalloc
+    const TreeStore* store = nullptr;  // the next batch's arrays are these (caller-owned); d_trees is the caller's too
 };
 
 // Room for `cap_trees` tree descriptors (forest_append fails beyond that).
@@ -352,6 +375,7 @@ struct IcpPending {
     int n_pairs;
     size_t h_off;   // first result of the batch in Ctx::h_icp_res
     int slot;       // index into Ctx::h_icp_passes
+    const sb_icp_result* d_res;  // the batch's results in device memory (arena), final once the stream reaches them
 };
 int icp_reserve_results(Ctx* ctx, size_t n_pairs);
 int icp_enqueue(Ctx* ctx, const Forest* f, const std::vector<PairDesc>& pairs, const sb_icp_config* cfg, IcpPending* out);
@@ -430,4 +454,26 @@ int loop_add_many(sb_loop* L, const double* xyz, const i64* offsets, int n_frame
 int loop_candidates_batch(sb_loop* L, const int* qslots, int n_q, std::vector<std::vector<std::pair<double, int>>>& cand,
                           std::vector<int>& total);
 int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* results, int* count);
+// loop_add for a cloud and descriptor already in device memory, in two steps: loop_add_enqueue grows the pools and
+// enqueues the device-to-device copies without waiting; loop_add_commit records the entry on the host once the stream
+// has run them.  Together they leave the state loop_add(cloud, frame_idx, desc) leaves; without the commit the
+// detector is unchanged (the copies land past its last committed entry).
+struct LoopAddPending {
+    int id, frame_idx;
+    i64 end_row;
+};
+int loop_add_enqueue(sb_loop* L, const double* d_xyz, i64 n, int frame_idx, const double* d_desc, LoopAddPending* out);
+void loop_add_commit(sb_loop* L, const LoopAddPending& p);
+
+// RAII entry guard of every C-ABI call: selects the device and resets the arena
+struct Enter {
+    Ctx* c;
+    explicit Enter(Ctx* ctx) : c(ctx) {
+        cudaSetDevice(c->device);
+        arena_reset(c);
+        c->tbuf_used = 0;  // everything the previous call enqueued has completed
+        c->err.clear();
+        c->n_ev = 0;
+    }
+};
 }  // namespace sb

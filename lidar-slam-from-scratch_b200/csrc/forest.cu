@@ -228,9 +228,22 @@ __global__ void __launch_bounds__(256) k_boxes_up(const TreeDesc* __restrict__ t
 // ---------------------------------------------------------------------------------------------------------------
 // host: build
 // ---------------------------------------------------------------------------------------------------------------
+void tree_store_need(i64 n, i64* boxes, i64* slots) {  // the layout loop of forest_append for one tree
+    i64 nb = 0, cnt = (n + 31) / 32;
+    while (true) {
+        nb += cnt;
+        if (cnt <= 32) break;
+        cnt = (cnt + 31) / 32;
+    }
+    int lg = 6;
+    while (((i64)1 << lg) < 2 * n) ++lg;
+    *boxes = nb;
+    *slots = (i64)1 << lg;
+}
+
 void forest_free(Forest* f) {
     if (!f) return;
-    if (!f->in_arena) {
+    if (!f->in_arena && !f->store) {
         // cudaFree only fails on a context that is already broken (a sticky error of an earlier kernel): it is recorded
         // for sb_last_error, there is nothing else to do with it while tearing down
         cudaError_t e = cudaSuccess;
@@ -316,7 +329,14 @@ int forest_append(Ctx* ctx, Forest* f, const double* d_xyz, const i64* h_off, co
     B.n_slots = n_slots;
     if (np >= (i64)0xffffffffLL) return fail(ctx, SB_ERR_RANGE, "index: more than 2^32-1 points in one batch of trees");
     size_t npa = (size_t)(np > 0 ? np : 1), nba = (size_t)(nb > 0 ? nb : 1);
-    if (f->in_arena) {
+    if (f->store) {
+        const TreeStore& S = *f->store;
+        if (!f->batches.empty() || np > S.cap_points || nb > S.cap_boxes || n_slots > S.cap_slots)
+            return fail(ctx, SB_ERR_CAPACITY, "forest: batch does not fit the caller's tree store");
+        B.pts = S.pts;
+        B.pts32 = S.pts32;
+        B.boxes = S.boxes;
+    } else if (f->in_arena) {
         SB_TRY(arena_get(ctx, npa, &B.pts));
         SB_TRY(arena_get(ctx, npa, &B.pts32));
         SB_TRY(arena_get(ctx, 6 * nba, &B.boxes));
@@ -722,7 +742,14 @@ int forest_normals(Ctx* ctx, Forest* f, int k, double* d_out_normals, double* d_
         return fail(ctx, SB_ERR_INVALID_ARG, "normals: every batch of a forest must use the same k");
     const size_t npa = (size_t)(B.n_points > 0 ? B.n_points : 1);
     const size_t nsa = (size_t)(B.n_slots > 0 ? B.n_slots : 1);
-    if (f->in_arena) {
+    if (f->store) {
+        const TreeStore& S = *f->store;
+        if (k > S.cap_k || B.n_slots > S.cap_slots || B.n_points > S.cap_points)
+            return fail(ctx, SB_ERR_CAPACITY, "normals: batch does not fit the caller's tree store");
+        B.normals = S.normals;
+        B.nbr = S.nbr;
+        B.grid = S.grid;
+    } else if (f->in_arena) {
         SB_TRY(arena_get(ctx, npa, &B.normals));
         SB_TRY(arena_get(ctx, npa * (size_t)k, &B.nbr));
         SB_TRY(arena_get(ctx, nsa, &B.grid));

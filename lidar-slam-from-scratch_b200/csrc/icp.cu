@@ -1077,6 +1077,7 @@ int icp_enqueue(Ctx* ctx, const Forest* f, const std::vector<PairDesc>& pairs_in
     out->n_pairs = n_pairs;
     out->h_off = ctx->icp_res_used;
     out->slot = -1;
+    out->d_res = nullptr;
     if (n_pairs == 0) return SB_OK;
     if (cfg->max_iterations < 0 || cfg->max_iterations > SB_MAX_ICP_ITERATIONS)
         return fail(ctx, SB_ERR_INVALID_ARG, "icp: max_iterations %d outside [0, %d]", cfg->max_iterations,
@@ -1137,6 +1138,7 @@ int icp_enqueue(Ctx* ctx, const Forest* f, const std::vector<PairDesc>& pairs_in
     job.n_items = n_items;
     job.pairs = d_pairs;
     job.results = d_res;
+    out->d_res = d_res;
     job.state = d_state;
     job.partials = d_part;
     job.queue = d_queue;

@@ -86,6 +86,48 @@ int loop_add(sb_loop* L, const double* xyz, i64 n, int frame_idx, const double* 
     return SB_OK;
 }
 
+// The streaming session's addFrame (odom.cu): the same pool layout as loop_add, with the cloud and the descriptor copied
+// device to device and no synchronise.  The host-side vectors change only in loop_add_commit.
+int loop_add_enqueue(sb_loop* L, const double* d_xyz, i64 n, int frame_idx, const double* d_desc, LoopAddPending* out) {
+    Ctx* ctx = L->ctx;
+    // the slot loop_add would use: a guest (non-owned former query) gives way
+    const size_t held = L->entry_id.size();
+    const size_t slots = held - (L->last_is_guest ? 1 : 0);
+    const i64 rows = L->cloud_off.empty() ? 0 : L->cloud_off[slots];
+    const int id = L->n_global;
+    SB_TRY(grow(L, &L->d_desc, &L->desc_cap, slots + 1, held, SB_SC_SIZE, FIRST_DESC_SLOTS));
+    SB_TRY(grow(L, &L->d_meta, &L->meta_cap, slots + 1, held, 1, FIRST_DESC_SLOTS));
+    const i64 held_rows = L->cloud_off.empty() ? 0 : L->cloud_off.back();
+    SB_TRY(grow(L, &L->d_clouds, &L->cloud_cap, (size_t)(rows + n), (size_t)held_rows, 3, FIRST_CLOUD_ROWS));
+    const int meta[2] = {frame_idx, id};
+    SB_TRY(table_upload(ctx, L->d_meta + slots, meta, sizeof(meta)));
+    if (n > 0)
+        SB_CUDA(ctx, cudaMemcpyAsync(L->d_clouds + 3 * rows, d_xyz, sizeof(double) * 3 * n, cudaMemcpyDeviceToDevice,
+                                     ctx->stream));
+    SB_CUDA(ctx, cudaMemcpyAsync(L->d_desc + slots * SB_SC_SIZE, d_desc, sizeof(double) * SB_SC_SIZE,
+                                 cudaMemcpyDeviceToDevice, ctx->stream));
+    out->id = id;
+    out->frame_idx = frame_idx;
+    out->end_row = rows + n;
+    return SB_OK;
+}
+
+void loop_add_commit(sb_loop* L, const LoopAddPending& p) {
+    if (L->last_is_guest) {
+        L->entry_id.pop_back();
+        L->frame_idx.pop_back();
+        L->cloud_off.pop_back();
+        L->last_is_guest = false;
+    }
+    if (L->cloud_off.empty()) L->cloud_off.push_back(0);
+    L->n_global = p.id + 1;
+    L->entry_id.push_back(p.id);
+    L->frame_idx.push_back(p.frame_idx);
+    L->cloud_off.push_back(p.end_row);
+    L->last_frame = p.frame_idx;
+    L->last_is_guest = (p.id % L->world) != L->rank;
+}
+
 // -------------------------------------------------------------------------------------------------------------
 // Candidate selection on the device (loop_closure.hpp:78-92: frame-gap filter, threshold, sort by (distance, entry)):
 // one block.  Every warp keeps the KSEL best (distance, entry) pairs of its share of the database in registers, entry

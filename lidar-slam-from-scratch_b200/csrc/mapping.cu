@@ -28,7 +28,7 @@ __global__ void __launch_bounds__(256) k_transform(const double* __restrict__ xy
     const double* T = poses + 16 * cloud_of(off, n_clouds, i);
     const double x = xyz[3 * i], y = xyz[3 * i + 1], z = xyz[3 * i + 2];
 #pragma unroll
-    for (int a = 0; a < 3; ++a) out[3 * i + a] = ((x * T[4 * a] + y * T[4 * a + 1]) + z * T[4 * a + 2]) + T[4 * a + 3];
+    for (int a = 0; a < 3; ++a) out[3 * i + a] = apply_row(T, a, x, y, z);
 }
 
 // update_occupancy_grid (slam_node.cpp:211-221) for world-frame rows: key = biased (x, y) cell, ~0 if filtered out

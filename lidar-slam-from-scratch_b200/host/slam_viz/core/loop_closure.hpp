@@ -84,6 +84,9 @@ public:
         return out;
     }
 
+    // extension: the underlying detector (b200::Odometry adds frames to it and runs its detect())
+    sb_loop* handle() const { return loop_.get(); }
+
 private:
     static LoopClosureResult result(const sb_loop_result& raw) {
         LoopClosureResult r;

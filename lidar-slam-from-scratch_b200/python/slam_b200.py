@@ -11,6 +11,7 @@ names and argument meaning to Python callers (tests, bench.py) on top of the C A
     ScanContext(cloud).distance(other)         scan_context.hpp:24-145
     LoopClosureDetector(cfg).addFrame/detect   loop_closure.hpp:41-149
     LoopClosureDetector.addFrames/detect_batch the same over a whole recorded sequence (slam_node.cpp:159-167)
+    Odometry(engine).push(scan, i)             SlamNode::process_frame one scan per call (slam_node.cpp:118-175)
 
 There is no CPU implementation here: if the shared library is missing, or no sm_100 device is usable, construction
 fails loudly.
@@ -64,6 +65,20 @@ class LoopResultC(C.Structure):
 class PoseFactorC(C.Structure):
     _fields_ = [("kind", C.c_int32), ("from_", C.c_int32), ("to", C.c_int32), ("pad", C.c_int32),
                 ("relative", C.c_double * 16), ("fitness", C.c_double), ("noise_scale", C.c_double)]
+
+
+class OdomConfigC(C.Structure):
+    _fields_ = [("voxel", C.c_double), ("min_points", C.c_int32), ("reserved", C.c_int32), ("max_error", C.c_double),
+                ("icp", ICPConfigC), ("initial_pose", C.c_double * 16)]
+
+
+class OdomFrameC(C.Structure):
+    _fields_ = [("frame_idx", C.c_int32), ("state", C.c_int32), ("n_points", C.c_int64), ("pose", C.c_double * 16),
+                ("icp", ICPResultC), ("n_loops", C.c_int32), ("pad", C.c_int32)]
+
+
+ODOM_ADD_FRAME, ODOM_DETECT = 1, 2
+ODOM_FIRST, ODOM_REGISTERED, ODOM_SKIPPED = 0, 1, 2
 
 
 FACTOR_DTYPE = np.dtype([("kind", "<i4"), ("from", "<i4"), ("to", "<i4"), ("pad", "<i4"), ("relative", "<f8", (4, 4)),
@@ -128,6 +143,16 @@ SYMBOLS = {
     "sb_loop_candidates_batch": (C.c_int, [_P, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
     "sb_loop_detect_batch": (C.c_int, [_P, _I32, C.c_int32, C.POINTER(LoopResultC), _I32]),
     "sb_odometry_poses": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_double, _D, _D]),
+    "sb_default_odom_config": (None, [C.POINTER(OdomConfigC)]),
+    "sb_odom_create": (C.c_int, [_P, C.POINTER(OdomConfigC), _P, C.POINTER(_P)]),
+    "sb_odom_free": (None, [_P]),
+    "sb_odom_reserve": (C.c_int, [_P, C.c_int64]),
+    "sb_odom_set_pose": (C.c_int, [_P, _D]),
+    "sb_odom_get_pose": (C.c_int, [_P, _D]),
+    "sb_odom_push": (C.c_int, [_P, _D, C.c_int64, C.c_int32, C.c_int32, C.POINTER(OdomFrameC), _D, C.POINTER(C.c_float),
+                               _D, C.POINTER(LoopResultC), C.c_int32]),
+    "sb_odom_push_f32": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(OdomFrameC), _D,
+                                   C.POINTER(C.c_float), _D, C.POINTER(LoopResultC), C.c_int32]),
     "sb_gather_results": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(ICPResultC), C.c_int32, C.POINTER(ICPResultC)]),
     "sb_gather_candidates": (C.c_int, [_P, _P, C.c_int32, _D, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
     "sb_odometry_factors": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_int32, C.c_double, C.POINTER(PoseFactorC)]),
@@ -719,3 +744,105 @@ class LoopClosureDetector:
         cnt = np.zeros(max(n, 1), dtype=np.int32)
         self.e._check(self.e.lib.sb_loop_detect_batch(self.h, q.ctypes.data_as(_I32), n, res, cnt.ctypes.data_as(_I32)))
         return [[self._result(res[i * m + j]) for j in range(cnt[i])] for i in range(n)]
+
+
+class OdomFrame:
+    """What Odometry.push returns for one frame: frame_idx, state (ODOM_FIRST / ODOM_REGISTERED / ODOM_SKIPPED),
+    n_points, pose (4x4), icp (ICPResult, registered frames only), loops (accepted loop closures, dicts as
+    LoopClosureDetector.detect returns them) and the outputs asked for: cloud (downsampled rows), world_f32
+    (PointCloud2 float32 xyz of the world-frame cloud), desc (Scan Context, 1200)."""
+
+    def __init__(self, f, loops, cloud, world_f32, desc):
+        self.frame_idx = int(f.frame_idx)
+        self.state = int(f.state)
+        self.n_points = int(f.n_points)
+        self.pose = np.array(f.pose[:]).reshape(4, 4)
+        self.icp = ICPResult(f.icp) if self.state == ODOM_REGISTERED else None
+        self.n_loops = int(f.n_loops)
+        self.loops = loops
+        self.cloud, self.world_f32, self.desc = cloud, world_f32, desc
+
+
+class Odometry:
+    """Streaming odometry session (sb_odom_*): SlamNode::process_frame (slam_node.cpp:118-175) one scan per call, with
+    the previous frame's cloud, index and normals kept on the device.  loop: an optional LoopClosureDetector on the same
+    engine, which must stay open while the session is."""
+
+    def __init__(self, engine, voxel=0.5, cfg=None, max_error=1.0, min_points=1000, initial_pose=None, loop=None):
+        self.e = engine
+        self.loop = loop
+        c = OdomConfigC()
+        engine.lib.sb_default_odom_config(C.byref(c))
+        c.voxel = float(voxel)
+        c.min_points = int(min_points)
+        c.max_error = float(max_error)
+        if cfg is not None:
+            c.icp = cfg
+        if initial_pose is not None:
+            c.initial_pose[:] = list(_f64(initial_pose).reshape(16))
+        self.cfg = c
+        h = _P()
+        engine._check(engine.lib.sb_odom_create(engine.h, C.byref(c), loop.h if loop is not None else None, C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.e.lib.sb_odom_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def reserve(self, max_raw_rows):
+        """Size every buffer for frames of up to max_raw_rows rows, so that no later push allocates."""
+        self.e._check(self.e.lib.sb_odom_reserve(self.h, int(max_raw_rows)))
+
+    def set_pose(self, pose):
+        """Continue the pose chain from `pose` (4x4), e.g. after a pose-graph optimisation (slam_node.cpp:177-185)."""
+        p = _f64(pose).reshape(16)
+        self.e._check(self.e.lib.sb_odom_set_pose(self.h, _dp(p)))
+
+    @property
+    def pose(self):
+        p = np.empty(16)
+        self.e._check(self.e.lib.sb_odom_get_pose(self.h, _dp(p)))
+        return p.reshape(4, 4)
+
+    def push(self, points, frame_idx, add_frame=True, detect=False, want_cloud=False, want_world_f32=False,
+             want_desc=False):
+        """One frame.  points: (n, 3) float64 rows, or float32 records (n, 3) / (n, 4) as read from PLY / KITTI files
+        (widened on the device).  add_frame adds the frame to the attached detector (ignored without one); detect runs
+        its detect() (needs a detector).  Returns an OdomFrame."""
+        f32 = isinstance(points, np.ndarray) and points.dtype == np.float32
+        if f32:
+            pts = np.ascontiguousarray(points)
+            if pts.ndim != 2:
+                raise ValueError("float32 points must be (n, 3) or (n, 4) records")
+        else:
+            pts = _f64(points, 3)
+        n = pts.shape[0]
+        flags = (ODOM_ADD_FRAME if add_frame and self.loop is not None else 0) | (ODOM_DETECT if detect else 0)
+        cloud = np.empty((max(n, 1), 3)) if want_cloud else None
+        world = np.empty((max(n, 1), 3), dtype=np.float32) if want_world_f32 else None
+        desc = np.empty(SB_SC_SIZE) if want_desc else None
+        cap = max(int(self.loop.cfg.max_candidates), 0) if (detect and self.loop is not None) else 0
+        loops = (LoopResultC * max(cap, 1))()
+        fr = OdomFrameC()
+        fp = C.POINTER(C.c_float)
+        args = (int(frame_idx), flags, C.byref(fr), _dp(cloud) if want_cloud else None,
+                world.ctypes.data_as(fp) if want_world_f32 else None, _dp(desc) if want_desc else None, loops, cap)
+        if f32:
+            s = self.e.lib.sb_odom_push_f32(self.h, _P(pts.ctypes.data), int(pts.shape[1]), n, *args)
+        else:
+            s = self.e.lib.sb_odom_push(self.h, _dp(pts), n, *args)
+        self.e._check(s)
+        m = int(fr.n_points)
+        state = int(fr.state)
+        out_cloud = cloud[:m].copy() if want_cloud else None
+        out_world = world[:m].copy() if (want_world_f32 and state != ODOM_SKIPPED) else None
+        out_desc = desc if (want_desc and state != ODOM_SKIPPED) else None
+        res = [LoopClosureDetector._result(loops[i]) for i in range(min(int(fr.n_loops), cap))]
+        return OdomFrame(fr, res, out_cloud, out_world, out_desc)
