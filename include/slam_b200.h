@@ -287,7 +287,7 @@ typedef struct sb_odom_frame {
     sb_icp_result icp;         /* state == SB_ODOM_REGISTERED, else zero                                             */
     int32_t n_loops, pad;      /* accepted loop closures (SB_ODOM_DETECT), counted like sb_loop_detect's *count       */
 } sb_odom_frame;
-/* xyz: n host fp64 rows.  Outputs (NULL: not wanted): out_xyz n_points*3 doubles (downsampled rows, sensor frame; also
+/* xyz: n host fp64 rows (pinned rows are copied without staging; a device pointer is SB_ERR_INVALID_ARG).  Outputs (NULL: not wanted): out_xyz n_points*3 doubles (downsampled rows, sensor frame; also
  * for a skipped frame), out_world_f32 n_points*3 floats and out_desc 1200 doubles (not for a skipped frame), loops: the
  * first min(n_loops, loop_capacity) accepted loop closures (NULL only with loop_capacity == 0).  The output buffers must
  * hold n rows: n_points is not known before the call. */

@@ -173,6 +173,19 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
         return fail(ctx, SB_ERR_INVALID_ARG, "odom: SB_ODOM_ADD_FRAME without a loop-closure detector");
     if ((flags & SB_ODOM_DETECT) && (!O->loop || O->loop->world != 1))
         return fail(ctx, SB_ERR_INVALID_ARG, "odom: SB_ODOM_DETECT needs a loop-closure detector with world == 1");
+    // the rows are host memory: pinned rows are copied as they are, anything else goes through pinned staging by
+    // memcpy, which a device address would crash
+    bool pinned = false;
+    if (n > 0) {
+        cudaPointerAttributes attr;
+        if (cudaPointerGetAttributes(&attr, xyz) == cudaSuccess) {
+            if (attr.type == cudaMemoryTypeDevice)
+                return fail(ctx, SB_ERR_INVALID_ARG, "odom: xyz is a device pointer; the session takes host rows");
+            pinned = attr.type == cudaMemoryTypeHost;
+        } else {
+            cudaGetLastError();
+        }
+    }
     memset(out, 0, sizeof(*out));
     out->frame_idx = frame_idx;
     memcpy(out->pose, O->pose, sizeof(O->pose));
@@ -186,9 +199,7 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
     SB_TRY(grow_dev(O, &O->d_raw, &O->raw_cap, std::max<i64>(in_bytes, 1)));
     if (n > 0) {
         const void* src = xyz;
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, xyz) != cudaSuccess || attr.type != cudaMemoryTypeHost) {
-            cudaGetLastError();
+        if (!pinned) {
             SB_TRY(grow_host(O, &O->h_in, &O->h_in_cap, in_bytes));
             memcpy(O->h_in, xyz, (size_t)in_bytes);
             src = O->h_in;

@@ -575,7 +575,8 @@ class KDTree:
 
     def close(self):
         if getattr(self, "h", None):
-            self.e.lib.sb_index_free(self.h)
+            if self.e.h:   # after Engine.close() its context is gone: freeing would touch it, so the handle is dropped
+                self.e.lib.sb_index_free(self.h)
             self.h = None
 
     def __del__(self):
@@ -651,7 +652,8 @@ class LoopClosureDetector:
 
     def close(self):
         if getattr(self, "h", None):
-            self.e.lib.sb_loop_free(self.h)
+            if self.e.h:   # after Engine.close() its context is gone: freeing would touch it, so the handle is dropped
+                self.e.lib.sb_loop_free(self.h)
             self.h = None
 
     def __del__(self):
@@ -787,7 +789,8 @@ class Odometry:
 
     def close(self):
         if getattr(self, "h", None):
-            self.e.lib.sb_odom_free(self.h)
+            if self.e.h:   # after Engine.close() its context is gone: freeing would touch it, so the handle is dropped
+                self.e.lib.sb_odom_free(self.h)
             self.h = None
 
     def __del__(self):
