@@ -341,6 +341,52 @@ int sb_global_map_f32(sb_ctx* ctx, const double* xyz, const int64_t* offsets, in
 int sb_odometry_poses(sb_ctx* ctx, const sb_icp_result* results, int32_t n, double max_error,
                       const double* initial_pose16, double* poses16_out);
 
+/* ---------------------------------------------------------------- device-resident map ---------------------- */
+/* The node's map state (slam_node.cpp:147-157, 177-238) kept in device memory: every keyframe's downsampled
+ * sensor-frame cloud and its pose (the node's downsampled_clouds_ and poses_), and the occupancy cell set.  A pose
+ * update after a loop closure uploads only the poses; the cell set, the global map and the world-frame window are
+ * rebuilt from the resident clouds.  A map belongs to one context.
+ * Every output equals the stateless entry point above on the resident clouds C and poses P, bit for bit, after any
+ * sequence of add / set_poses: sb_map_occupancy_cells = sb_occupancy_cells(C, P, grid), sb_map_global[_f32] =
+ * sb_global_map[_f32](C, P, voxel), sb_map_world_f32 = sb_transform_clouds_f32 of the listed entries.
+ * A call that fails leaves the map as it was: a non-finite row or pose, or a cell index that does not fit an int,
+ * is SB_ERR_RANGE. */
+typedef struct sb_map sb_map;
+/* grid: NULL -> sb_default_grid_config */
+int sb_map_create(sb_ctx* ctx, const sb_grid_config* grid, sb_map** out);
+void sb_map_free(sb_map* map);
+/* Optional: room for n_entries entries, total_rows rows and n_cells occupancy cells, so that no later call allocates
+ * while the map stays within them.  Without it the buffers start small and double. */
+int sb_map_reserve(sb_map* map, int64_t n_entries, int64_t total_rows, int64_t n_cells);
+int64_t sb_map_size(const sb_map* map);          /* entries */
+int64_t sb_map_rows(const sb_map* map);          /* rows over all entries: what sb_map_global's output must hold */
+/* Measurement hook: [0] entries, [1] rows, [2] cell-table slots the device buffers hold now */
+int sb_map_capacity(const sb_map* map, int64_t* caps3);
+int sb_map_clear(sb_map* map);
+/* One entry: a sensor-frame cloud (n host fp64 rows, n may be 0) and its pose (row-major 4x4); its cells are inserted
+ * at once (update_occupancy_grid, slam_node.cpp:152, 211-221). */
+int sb_map_add(sb_map* map, const double* xyz, int64_t n, const double* pose16);
+/* The poses of entries [first, first + n) replaced (PoseGraph::getAllPoses after optimize, slam_node.cpp:177-185);
+ * the cell set is rebuilt on the device from every resident cloud (rebuild_occupancy_grid, slam_node.cpp:222-229). */
+int sb_map_set_poses(sb_map* map, int32_t first, int32_t n, const double* poses16);
+int sb_map_get_poses(const sb_map* map, int32_t first, int32_t n, double* poses16);
+/* The cells, ascending in (x, y), 2 ints each, up to `capacity`; *out_count = all of them. */
+int sb_map_occupancy_cells(sb_map* map, int32_t* out_cells, int64_t capacity, int64_t* out_count);
+/* Entries [first, first + n) in the world frame as PointCloud2 float32 records (the node's window of the last 20
+ * world clouds, publish_current_scan): *out_rows rows; out_xyz must hold them. */
+int sb_map_world_f32(sb_map* map, int32_t first, int32_t n, float* out_xyz, int64_t* out_rows);
+/* All entries in the world frame, voxel grid at `voxel` (<= 0: the concatenation), as fp64 rows or float32 records
+ * (publish_global_map, slam_node.cpp:196-209, 235-238).  out_xyz must hold sb_map_rows rows. */
+int sb_map_global(sb_map* map, double voxel, double* out_xyz, int64_t* out_m);
+int sb_map_global_f32(sb_map* map, double voxel, float* out_xyz, int64_t* out_m);
+
+/* A streaming session that also feeds a map (sb_odom_create for map == NULL).  With SB_ODOM_ADD_MAP a push adds the
+ * frame to the map: its downsampled rows (copied device to device) and its pose; a SKIPPED frame adds an entry with no
+ * rows and the repeated pose, so that map entry i is the node's poses_[i].  The map must be created on ctx and must
+ * outlive the session.  A push that fails leaves the map as it was too. */
+enum { SB_ODOM_ADD_MAP = 4 };
+int sb_odom_create2(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_map* map, sb_odom** out);
+
 /* ---------------------------------------------------------------- multi-GPU exchanges (SURVEY.md 8e) -------- */
 /* One process per GPU; the caller owns the NCCL communicator (an ncclComm_t passed as void*; NCCL itself is looked up
  * in the already-loaded libnccl.so.2 at first use, it is not a link dependency of this library).  The reference has no

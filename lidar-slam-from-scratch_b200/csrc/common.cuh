@@ -191,6 +191,35 @@ __device__ __forceinline__ unsigned lanemask_lt() {
 // error flag bits written to Ctx::d_flags
 enum { FLAG_NONFINITE = 1, FLAG_KEY_RANGE = 2 };
 
+#ifdef __CUDACC__
+// cloud of row i of a CSR point set (offsets ascending, offsets[0] <= i; an empty cloud never owns a row)
+__device__ __forceinline__ int cloud_of(const i64* __restrict__ off, int n_clouds, i64 i) {
+    int lo = 0, hi = n_clouds;
+    while (hi - lo > 1) {
+        int mid = (lo + hi) >> 1;
+        if (off[mid] <= i) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// update_occupancy_grid (slam_node.cpp:211-221) for one world-frame row of a cloud whose pose translation is (tx, ty):
+// the biased (x, y) cell key, ascending in (x, y) as an unsigned integer; ~0 if the row is filtered out (*out_of_range
+// set if its cell index does not fit an int).  The one expression of mapping.cu's k_occ_keys and map.cu's
+// k_map_occ_insert, so both cell sets hold the same keys.
+__device__ __forceinline__ u64 occ_key(double x, double y, double z, double tx, double ty, double res, double hmin,
+                                       double hmax, double max_range, bool* out_of_range) {
+    if (z < hmin || z > hmax) return ~0ull;   // NaN z passes both tests like the reference's comparisons
+    const double dx = x - tx, dy = y - ty;
+    const double r = sqrt(dx * dx + dy * dy);
+    if (r > max_range || r < 0.5) return ~0ull;
+    const double cx = floor(__ddiv_rn(x, res)), cy = floor(__ddiv_rn(y, res));
+    if (fabs(cx) < 2147483647.0 && fabs(cy) < 2147483647.0)
+        return ((u64)(uint32_t)((int)cx ^ 0x80000000) << 32) | (u64)(uint32_t)((int)cy ^ 0x80000000);
+    *out_of_range = true;  // static_cast<int> of such a value is undefined in the reference
+    return ~0ull;
+}
+#endif
+
 // ---------------------------------------------------------------------------------------------------------------
 // scan_sort.cu
 // ---------------------------------------------------------------------------------------------------------------
@@ -464,6 +493,42 @@ struct LoopAddPending {
 };
 int loop_add_enqueue(sb_loop* L, const double* d_xyz, i64 n, int frame_idx, const double* d_desc, LoopAddPending* out);
 void loop_add_commit(sb_loop* L, const LoopAddPending& p);
+}  // namespace sb
+
+// map.cu — device-resident keyframe map: every entry's sensor-frame rows and pose, and the occupancy cell set
+struct sb_map {
+    sb::Ctx* ctx = nullptr;
+    sb_grid_config grid;
+    std::vector<sb::i64> off{0};     // host CSR of the entries' rows, entries + 1
+    std::vector<double> poses;       // host copy of the poses, 16 per entry
+    double* d_rows = nullptr;        // rows x 3 (fp64, sensor frame)
+    sb::i64 row_cap = 0;             // in rows
+    sb::i64* d_off = nullptr;        // device copy of off
+    double* d_poses = nullptr;       // 16 per entry
+    sb::i64 entry_cap = 0;           // entries d_off / d_poses hold
+    unsigned long long* d_table = nullptr;   // open-addressing set of cell keys, ~0 = empty slot
+    sb::i64 table_cap = 0;           // slots, a power of two
+    sb::i64 n_cells = 0;             // keys in the table
+    unsigned long long* d_stat = nullptr;    // [0] keys a launch inserted, [1] flag bits (FLAG_*)
+    unsigned long long* h_stat = nullptr;    // pinned copy of d_stat
+    bool pending = false;            // an add was enqueued and not finished: the table may hold its cells
+    std::vector<void*> retired;      // outgrown buffers, released with the map
+};
+
+namespace sb {
+// The streaming session's half of sb_map_add (odom.cu): the frame's rows and pose, already in device memory, are copied
+// device to device and its cells are inserted, without a synchronise.  After the caller's synchronise, map_add_finish
+// records the entry; if the insert failed it restores the cell set from the committed entries and returns the error,
+// and the map is as it was.
+struct MapAddPending {
+    i64 end_row;
+};
+int map_add_enqueue(sb_map* M, const double* d_xyz, i64 n, const double* d_pose, MapAddPending* out);
+int map_add_finish(sb_map* M, const MapAddPending& p, const double* pose16);
+// after a failed call that enqueued an add without finishing it: the cell set of the committed entries again
+int map_add_abort(sb_map* M);
+// sb_map_add: host rows and pose, one synchronise (the session adds a skipped frame this way: no rows, the same pose)
+int map_add(sb_map* M, const double* xyz, i64 n, const double* pose16);
 
 // RAII entry guard of every C-ABI call: selects the device and resets the arena
 struct Enter {

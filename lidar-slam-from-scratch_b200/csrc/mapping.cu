@@ -9,16 +9,6 @@
 
 namespace sb {
 
-// cloud of row i (offsets ascending, offsets[0] <= i)
-__device__ __forceinline__ int cloud_of(const i64* __restrict__ off, int n_clouds, i64 i) {
-    int lo = 0, hi = n_clouds;
-    while (hi - lo > 1) {
-        int mid = (lo + hi) >> 1;
-        if (off[mid] <= i) lo = mid; else hi = mid;
-    }
-    return lo;
-}
-
 // out = p * R^T + t with the association of Transformation::apply (types.hpp:110-115)
 __global__ void __launch_bounds__(256) k_transform(const double* __restrict__ xyz, const i64* __restrict__ off,
                                                    int n_clouds, const double* __restrict__ poses, i64 n,
@@ -39,21 +29,10 @@ __global__ void __launch_bounds__(256) k_occ_keys(const double* __restrict__ wor
     const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const double* T = poses + 16 * cloud_of(off, n_clouds, i);
-    const double x = world[3 * i], y = world[3 * i + 1], z = world[3 * i + 2];
-    u64 key = ~0ull;
-    if (!(z < hmin || z > hmax)) {  // NaN z passes both tests like the reference's comparisons
-        const double dx = x - T[3], dy = y - T[7];
-        const double r = sqrt(dx * dx + dy * dy);
-        if (!(r > max_range || r < 0.5)) {
-            const double cx = floor(__ddiv_rn(x, res)), cy = floor(__ddiv_rn(y, res));
-            if (fabs(cx) < 2147483647.0 && fabs(cy) < 2147483647.0) {
-                key = ((u64)(uint32_t)((int)cx ^ 0x80000000) << 32) | (u64)(uint32_t)((int)cy ^ 0x80000000);
-            } else {
-                atomicOr(flags, FLAG_KEY_RANGE);  // static_cast<int> of such a value is undefined in the reference
-            }
-        }
-    }
-    keys[i] = key;
+    bool out_of_range = false;
+    keys[i] = occ_key(world[3 * i], world[3 * i + 1], world[3 * i + 2], T[3], T[7], res, hmin, hmax, max_range,
+                      &out_of_range);
+    if (out_of_range) atomicOr(flags, FLAG_KEY_RANGE);
     vals[i] = (uint32_t)i;
 }
 

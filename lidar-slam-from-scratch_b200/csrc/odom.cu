@@ -81,6 +81,7 @@ struct sb_odom {
     Ctx* ctx = nullptr;
     sb_odom_config cfg;
     sb_loop* loop = nullptr;
+    sb_map* map = nullptr;      // SB_ODOM_ADD_MAP
     OdomSlot slot[2];
     int prev = -1;              // slot of the previous (committed) frame; -1 before the first
     double pose[16];            // host copy of the committed pose
@@ -168,7 +169,9 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
     if (stride < 3) return fail(ctx, SB_ERR_INVALID_ARG, "odom: row stride %d < 3", stride);
     if (loop_capacity < 0 || (loop_capacity > 0 && !loops))
         return fail(ctx, SB_ERR_INVALID_ARG, "odom: loops may be NULL only with loop_capacity 0");
-    if (flags & ~(SB_ODOM_ADD_FRAME | SB_ODOM_DETECT)) return fail(ctx, SB_ERR_INVALID_ARG, "odom: unknown flags %d", flags);
+    if (flags & ~(SB_ODOM_ADD_FRAME | SB_ODOM_DETECT | SB_ODOM_ADD_MAP))
+        return fail(ctx, SB_ERR_INVALID_ARG, "odom: unknown flags %d", flags);
+    if ((flags & SB_ODOM_ADD_MAP) && !O->map) return fail(ctx, SB_ERR_INVALID_ARG, "odom: SB_ODOM_ADD_MAP without a map");
     if ((flags & SB_ODOM_ADD_FRAME) && !O->loop)
         return fail(ctx, SB_ERR_INVALID_ARG, "odom: SB_ODOM_ADD_FRAME without a loop-closure detector");
     if ((flags & SB_ODOM_DETECT) && (!O->loop || O->loop->world != 1))
@@ -226,6 +229,8 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
             SB_CUDA(ctx, cudaMemcpyAsync(out_xyz, S.xyz, sizeof(double) * 3 * m, cudaMemcpyDeviceToHost, ctx->stream));
             SB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         }
+        // the map keeps one entry per pose of the node (poses_): no rows, the pose repeated
+        if (flags & SB_ODOM_ADD_MAP) SB_TRY(map_add(O->map, nullptr, 0, O->pose));
         return SB_OK;
     }
     if (m == 0) return fail(ctx, SB_ERR_EMPTY, "odom: empty frame (undefined behaviour in the reference, kdtree.hpp:25,119)");
@@ -286,6 +291,10 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
     const bool add = (flags & SB_ODOM_ADD_FRAME) != 0;
     LoopAddPending LP;
     if (add) SB_TRY(loop_add_enqueue(O->loop, S.xyz, m, frame_idx, d_desc, &LP));
+    // 7b. the map's entry (update_occupancy_grid, slam_node.cpp:152): rows and pose device to device, cells inserted
+    const bool add_map = (flags & SB_ODOM_ADD_MAP) != 0;
+    MapAddPending MP;
+    if (add_map) SB_TRY(map_add_enqueue(O->map, S.xyz, m, O->d_pose + 16 * (1 - O->pi), &MP));
     // 8. one copy of the outputs back, and the frame's final synchronise (icp_collect waits for the stream)
     const size_t d2h = (out_xyz || out_world_f32 || out_desc) ? o_end : OUT_DESC;
     SB_CUDA(ctx, cudaMemcpyAsync(O->h_out, O->d_out, d2h, cudaMemcpyDeviceToHost, ctx->stream));
@@ -298,6 +307,8 @@ int push_impl(sb_odom* O, const void* xyz, int f32, int stride, i64 n, int32_t f
     trace_mark(ctx, "odom:end");
     trace_dump(ctx);
 
+    // the map's entry first: a map whose insert fails restores itself, and the push fails before anything else commits
+    if (add_map) SB_TRY(map_add_finish(O->map, MP, reinterpret_cast<const double*>(O->h_out)));
     // commit: this frame becomes the previous one
     if (add) loop_add_commit(O->loop, LP);
     S.tree = F.h_trees[1];
@@ -332,8 +343,16 @@ int push_entry(sb_odom* O, const void* xyz, int f32, int stride, int64_t n, int3
     Enter g(O->ctx);
     const int s = push_impl(O, xyz, f32, stride, (i64)n, frame_idx, flags, out, out_xyz, out_world_f32, out_desc, loops,
                             loop_capacity);
-    // a failed push may leave copies or kernels in flight: the next call reuses the staging buffers and the arena
-    if (s != SB_OK) cudaStreamSynchronize(O->ctx->stream);
+    // a failed push may leave copies or kernels in flight: the next call reuses the staging buffers and the arena; a map
+    // add it enqueued but did not finish is taken back
+    if (s != SB_OK) {
+        cudaStreamSynchronize(O->ctx->stream);
+        if (O->map && O->map->pending) {
+            const std::string msg = O->ctx->err;
+            map_add_abort(O->map);
+            O->ctx->err = msg;
+        }
+    }
     return s;
 }
 
@@ -352,11 +371,16 @@ void sb_default_odom_config(sb_odom_config* cfg) {
 }
 
 int sb_odom_create(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_odom** out) {
+    return sb_odom_create2(ctx, cfg, loop, nullptr, out);
+}
+
+int sb_odom_create2(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_map* map, sb_odom** out) {
     if (!ctx || !cfg || !out) return SB_ERR_INVALID_ARG;
     *out = nullptr;
     Ctx* c = &ctx->c;
     Enter g(c);
     if (loop && loop->ctx != c) return fail(c, SB_ERR_INVALID_ARG, "odom: the loop-closure detector belongs to another context");
+    if (map && map->ctx != c) return fail(c, SB_ERR_INVALID_ARG, "odom: the map belongs to another context");
     if (cfg->icp.normals_k < 1 || cfg->icp.normals_k > SB_MAX_K)
         return fail(c, SB_ERR_INVALID_ARG, "odom: normals_k %d outside [1, %d]", cfg->icp.normals_k, SB_MAX_K);
     if (cfg->icp.max_iterations < 0 || cfg->icp.max_iterations > SB_MAX_ICP_ITERATIONS)
@@ -366,6 +390,7 @@ int sb_odom_create(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_odo
     O->ctx = c;
     O->cfg = *cfg;
     O->loop = loop;
+    O->map = map;
     memcpy(O->pose, cfg->initial_pose, sizeof(O->pose));
     int s = SB_OK;
     if (cudaMalloc(&O->d_pose, sizeof(double) * 32) != cudaSuccess ||

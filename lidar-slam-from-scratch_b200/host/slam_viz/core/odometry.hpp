@@ -1,13 +1,15 @@
 // odometry.hpp — extension (not a reference name): SlamNode::process_frame (slam_node.cpp:118-175) as one call per
 // frame over the streaming session of the C ABI (sb_odom_*).  The previous frame's cloud, index and normals stay on the
 // device; the frame is uploaded once.  Results come back as the reference's types (ICPResult, Transformation,
-// LoopClosureResult), and frames can go to an existing LoopClosureDetector, which must outlive the session.
+// LoopClosureResult), and frames can go to an existing LoopClosureDetector and an existing Map, which must outlive the
+// session.
 #pragma once
 #include <memory>
 #include <vector>
 
 #include "icp.hpp"
 #include "loop_closure.hpp"
+#include "map.hpp"
 
 namespace slam {
 namespace b200 {
@@ -33,8 +35,9 @@ struct OdometryFrame {
 
 class Odometry {
 public:
-    explicit Odometry(const OdometryConfig& config = OdometryConfig(), LoopClosureDetector* loop = nullptr)
-        : loop_(loop) {
+    explicit Odometry(const OdometryConfig& config = OdometryConfig(), LoopClosureDetector* loop = nullptr,
+                      Map* map = nullptr)
+        : loop_(loop), map_(map) {
         sb_odom_config c;
         sb_default_odom_config(&c);
         c.voxel = config.voxel_size;
@@ -46,7 +49,8 @@ public:
         config.icp.initial_transform.to_row_major(c.icp.initial_transform);
         config.initial_pose.to_row_major(c.initial_pose);
         sb_odom* o = nullptr;
-        check(sb_odom_create(context(), &c, loop ? loop->handle() : nullptr, &o), "Odometry");
+        check(sb_odom_create2(context(), &c, loop ? loop->handle() : nullptr, map ? map->handle() : nullptr, &o),
+              "Odometry");
         odom_ = std::shared_ptr<sb_odom>(o, [](sb_odom* p) { sb_odom_free(p); });
     }
 
@@ -64,9 +68,12 @@ public:
 
     // One scan (raw rows).  add_frame: LoopClosureDetector::addFrame of the downsampled frame (slam_node.cpp:159);
     // detect: its detect() right after (slam_node.cpp:160-167).  Both need the detector given at construction.
-    OdometryFrame push(const PointCloud& scan, int frame_idx, bool add_frame = true, bool detect = false) {
+    // add_map: the frame goes to the map given at construction (a skipped frame as an entry with no rows).
+    OdometryFrame push(const PointCloud& scan, int frame_idx, bool add_frame = true, bool detect = false,
+                       bool add_map = true) {
         const int64_t n = (int64_t)scan.size();
-        const int flags = (add_frame && loop_ ? SB_ODOM_ADD_FRAME : 0) | (detect ? SB_ODOM_DETECT : 0);
+        const int flags = (add_frame && loop_ ? SB_ODOM_ADD_FRAME : 0) | (detect ? SB_ODOM_DETECT : 0) |
+                          (add_map && map_ ? SB_ODOM_ADD_MAP : 0);
         PointCloud::Matrix cloud(n, 3);
         std::vector<float> world((size_t)(3 * (n > 0 ? n : 1)));
         std::vector<sb_loop_result> raw((size_t)max_loops_);
@@ -103,6 +110,7 @@ public:
 
 private:
     LoopClosureDetector* loop_;
+    Map* map_;
     std::shared_ptr<sb_odom> odom_;
     static constexpr int max_loops_ = 64;   // accepted loops returned per frame (the node's config accepts 3)
 };

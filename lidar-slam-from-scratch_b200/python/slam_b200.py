@@ -12,6 +12,7 @@ names and argument meaning to Python callers (tests, bench.py) on top of the C A
     LoopClosureDetector(cfg).addFrame/detect   loop_closure.hpp:41-149
     LoopClosureDetector.addFrames/detect_batch the same over a whole recorded sequence (slam_node.cpp:159-167)
     Odometry(engine).push(scan, i)             SlamNode::process_frame one scan per call (slam_node.cpp:118-175)
+    Map(engine).add / set_poses / ...          the node's keyframe clouds, poses and occupancy grid on the device
 
 There is no CPU implementation here: if the shared library is missing, or no sm_100 device is usable, construction
 fails loudly.
@@ -77,7 +78,7 @@ class OdomFrameC(C.Structure):
                 ("icp", ICPResultC), ("n_loops", C.c_int32), ("pad", C.c_int32)]
 
 
-ODOM_ADD_FRAME, ODOM_DETECT = 1, 2
+ODOM_ADD_FRAME, ODOM_DETECT, ODOM_ADD_MAP = 1, 2, 4
 ODOM_FIRST, ODOM_REGISTERED, ODOM_SKIPPED = 0, 1, 2
 
 
@@ -153,6 +154,21 @@ SYMBOLS = {
                                _D, C.POINTER(LoopResultC), C.c_int32]),
     "sb_odom_push_f32": (C.c_int, [_P, _P, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.POINTER(OdomFrameC), _D,
                                    C.POINTER(C.c_float), _D, C.POINTER(LoopResultC), C.c_int32]),
+    "sb_map_create": (C.c_int, [_P, _P, C.POINTER(_P)]),
+    "sb_map_free": (None, [_P]),
+    "sb_map_reserve": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int64]),
+    "sb_map_size": (C.c_int64, [_P]),
+    "sb_map_rows": (C.c_int64, [_P]),
+    "sb_map_capacity": (C.c_int, [_P, _I64]),
+    "sb_map_clear": (C.c_int, [_P]),
+    "sb_map_add": (C.c_int, [_P, _D, C.c_int64, _D]),
+    "sb_map_set_poses": (C.c_int, [_P, C.c_int32, C.c_int32, _D]),
+    "sb_map_get_poses": (C.c_int, [_P, C.c_int32, C.c_int32, _D]),
+    "sb_map_occupancy_cells": (C.c_int, [_P, _I32, C.c_int64, _I64]),
+    "sb_map_world_f32": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_float), _I64]),
+    "sb_map_global": (C.c_int, [_P, C.c_double, _D, _I64]),
+    "sb_map_global_f32": (C.c_int, [_P, C.c_double, C.POINTER(C.c_float), _I64]),
+    "sb_odom_create2": (C.c_int, [_P, C.POINTER(OdomConfigC), _P, _P, C.POINTER(_P)]),
     "sb_gather_results": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(ICPResultC), C.c_int32, C.POINTER(ICPResultC)]),
     "sb_gather_candidates": (C.c_int, [_P, _P, C.c_int32, _D, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
     "sb_odometry_factors": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_int32, C.c_double, C.POINTER(PoseFactorC)]),
@@ -767,12 +783,14 @@ class OdomFrame:
 
 class Odometry:
     """Streaming odometry session (sb_odom_*): SlamNode::process_frame (slam_node.cpp:118-175) one scan per call, with
-    the previous frame's cloud, index and normals kept on the device.  loop: an optional LoopClosureDetector on the same
-    engine, which must stay open while the session is."""
+    the previous frame's cloud, index and normals kept on the device.  loop: an optional LoopClosureDetector, map: an
+    optional Map, both on the same engine and open while the session is."""
 
-    def __init__(self, engine, voxel=0.5, cfg=None, max_error=1.0, min_points=1000, initial_pose=None, loop=None):
+    def __init__(self, engine, voxel=0.5, cfg=None, max_error=1.0, min_points=1000, initial_pose=None, loop=None,
+                 map=None):
         self.e = engine
         self.loop = loop
+        self.map = map
         c = OdomConfigC()
         engine.lib.sb_default_odom_config(C.byref(c))
         c.voxel = float(voxel)
@@ -784,7 +802,8 @@ class Odometry:
             c.initial_pose[:] = list(_f64(initial_pose).reshape(16))
         self.cfg = c
         h = _P()
-        engine._check(engine.lib.sb_odom_create(engine.h, C.byref(c), loop.h if loop is not None else None, C.byref(h)))
+        engine._check(engine.lib.sb_odom_create2(engine.h, C.byref(c), loop.h if loop is not None else None,
+                                                 map.h if map is not None else None, C.byref(h)))
         self.h = h
 
     def close(self):
@@ -815,10 +834,11 @@ class Odometry:
         return p.reshape(4, 4)
 
     def push(self, points, frame_idx, add_frame=True, detect=False, want_cloud=False, want_world_f32=False,
-             want_desc=False):
+             want_desc=False, add_map=True):
         """One frame.  points: (n, 3) float64 rows, or float32 records (n, 3) / (n, 4) as read from PLY / KITTI files
         (widened on the device).  add_frame adds the frame to the attached detector (ignored without one); detect runs
-        its detect() (needs a detector).  Returns an OdomFrame."""
+        its detect() (needs a detector); add_map adds the frame to the attached map (ignored without one: a skipped
+        frame as an entry with no rows and the repeated pose).  Returns an OdomFrame."""
         f32 = isinstance(points, np.ndarray) and points.dtype == np.float32
         if f32:
             pts = np.ascontiguousarray(points)
@@ -827,7 +847,8 @@ class Odometry:
         else:
             pts = _f64(points, 3)
         n = pts.shape[0]
-        flags = (ODOM_ADD_FRAME if add_frame and self.loop is not None else 0) | (ODOM_DETECT if detect else 0)
+        flags = ((ODOM_ADD_FRAME if add_frame and self.loop is not None else 0) | (ODOM_DETECT if detect else 0) |
+                 (ODOM_ADD_MAP if add_map and self.map is not None else 0))
         cloud = np.empty((max(n, 1), 3)) if want_cloud else None
         world = np.empty((max(n, 1), 3), dtype=np.float32) if want_world_f32 else None
         desc = np.empty(SB_SC_SIZE) if want_desc else None
@@ -849,3 +870,116 @@ class Odometry:
         out_desc = desc if (want_desc and state != ODOM_SKIPPED) else None
         res = [LoopClosureDetector._result(loops[i]) for i in range(min(int(fr.n_loops), cap))]
         return OdomFrame(fr, res, out_cloud, out_world, out_desc)
+
+
+class Map:
+    """Device-resident map (sb_map_*): the node's keyframe clouds (sensor frame), their poses and the occupancy cell set
+    (slam_node.cpp:147-157, 177-238).  After a pose-graph optimisation only the poses are uploaded (set_poses); the
+    cells, the global map and the world-frame window are rebuilt from the resident clouds, with the bits of
+    Engine.occupancy_cells / global_map / transform_clouds_f32 over the same clouds and poses."""
+
+    def __init__(self, engine, resolution=0.2, height_min=0.3, height_max=2.0, max_range=40.0):
+        self.e = engine
+        self.grid = (C.c_double * 4)(resolution, height_min, height_max, max_range)
+        h = _P()
+        engine._check(engine.lib.sb_map_create(engine.h, C.cast(self.grid, _P), C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            if self.e.h:   # after Engine.close() its context is gone: freeing would touch it, so the handle is dropped
+                self.e.lib.sb_map_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def reserve(self, n_entries, total_rows, n_cells):
+        """Room for n_entries entries, total_rows rows and n_cells cells: no later call allocates within them."""
+        self.e._check(self.e.lib.sb_map_reserve(self.h, int(n_entries), int(total_rows), int(n_cells)))
+
+    def size(self):
+        return int(self.e.lib.sb_map_size(self.h))
+
+    def __len__(self):
+        return self.size()
+
+    @property
+    def rows(self):
+        return int(self.e.lib.sb_map_rows(self.h))
+
+    def capacity(self):
+        """(entries, rows, cell-table slots) the device buffers hold now."""
+        c = np.zeros(3, dtype=np.int64)
+        self.e._check(self.e.lib.sb_map_capacity(self.h, c.ctypes.data_as(_I64)))
+        return tuple(int(v) for v in c)
+
+    def clear(self):
+        self.e._check(self.e.lib.sb_map_clear(self.h))
+
+    def add(self, points, pose):
+        """One entry: a sensor-frame cloud (n, 3) and its 4x4 pose; its occupancy cells are inserted at once."""
+        p = _f64(points, 3)
+        T = _f64(pose)
+        if T.size != 16:
+            raise ValueError("pose must be a 4x4 matrix")
+        self.e._check(self.e.lib.sb_map_add(self.h, _dp(p), p.shape[0], _dp(T.reshape(16))))
+
+    def _range(self, first, n):
+        first, n = int(first), int(n)
+        if first < 0 or n < 0 or first + n > self.size():
+            raise ValueError(f"entries [{first}, {first + n}) outside [0, {self.size()})")
+        return first, n
+
+    def set_poses(self, poses, first=0):
+        """Replace the poses of entries [first, first + len(poses)) ((k, 4, 4)); the cell set is rebuilt on the device."""
+        T = _f64(poses)
+        if T.size % 16:
+            raise ValueError("poses must be (k, 4, 4)")
+        T = T.reshape(-1, 16)
+        first, n = self._range(first, T.shape[0])
+        self.e._check(self.e.lib.sb_map_set_poses(self.h, first, n, _dp(T)))
+
+    def poses(self, first=0, n=None):
+        first, n = self._range(first, self.size() - int(first) if n is None else n)
+        out = np.empty((max(n, 1), 16))
+        self.e._check(self.e.lib.sb_map_get_poses(self.h, first, n, _dp(out)))
+        return out[:n].reshape(n, 4, 4)
+
+    def occupancy_cells(self, capacity=None):
+        """(cells (m, 2) int32 ascending in (x, y), count): the first `capacity` cells (all by default) and how many
+        there are."""
+        if capacity is None:
+            cnt = C.c_int64(0)
+            self.e._check(self.e.lib.sb_map_occupancy_cells(self.h, None, 0, C.byref(cnt)))
+            capacity = cnt.value
+        cap = int(capacity)
+        if cap < 0:
+            raise ValueError("capacity must be >= 0")
+        cells = np.empty((max(cap, 1), 2), dtype=np.int32)
+        cnt = C.c_int64(0)
+        self.e._check(self.e.lib.sb_map_occupancy_cells(self.h, cells.ctypes.data_as(_I32), cap, C.byref(cnt)))
+        return cells[:min(cnt.value, cap)].copy(), int(cnt.value)
+
+    def world_f32(self, first, n):
+        """Entries [first, first + n) in the world frame as PointCloud2 float32 xyz records."""
+        first, n = self._range(first, n)
+        out = np.empty((max(self.rows, 1), 3), dtype=np.float32)
+        m = C.c_int64(0)
+        self.e._check(self.e.lib.sb_map_world_f32(self.h, first, n, out.ctypes.data_as(C.POINTER(C.c_float)),
+                                                  C.byref(m)))
+        return out[:m.value].copy()
+
+    def global_map(self, voxel, f32=False):
+        """All entries in the world frame, voxel grid at `voxel` (<= 0: the concatenation); float32 records if f32."""
+        out = np.empty((max(self.rows, 1), 3), dtype=np.float32 if f32 else np.float64)
+        m = C.c_int64(0)
+        if f32:
+            s = self.e.lib.sb_map_global_f32(self.h, float(voxel), out.ctypes.data_as(C.POINTER(C.c_float)), C.byref(m))
+        else:
+            s = self.e.lib.sb_map_global(self.h, float(voxel), _dp(out), C.byref(m))
+        self.e._check(s)
+        return out[:m.value].copy()
