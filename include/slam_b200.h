@@ -387,6 +387,30 @@ int sb_map_global_f32(sb_map* map, double voxel, float* out_xyz, int64_t* out_m)
 enum { SB_ODOM_ADD_MAP = 4 };
 int sb_odom_create2(sb_ctx* ctx, const sb_odom_config* cfg, sb_loop* loop, sb_map* map, sb_odom** out);
 
+/* ---------------------------------------------------------------- many streaming sessions in one call ------ */
+/* One frame into each of n sessions (SB_ODOM_* semantics per session), with one voxel grid, one index build and one ICP
+ * batch for all of them: many live streams (a fleet of robots, several LiDARs, replayed sequences) on one GPU.  The
+ * result is exactly what n calls of sb_odom_push would give, in array order: every output and every session, detector
+ * and map state afterwards, bit for bit; single and many pushes may be mixed on the same sessions.  Arrays are indexed
+ * by session: xyz[i] holds n_rows[i] rows, out[i] receives the frame, and out_xyz[i], out_world_f32[i], out_desc[i],
+ * loops[i] / loop_capacity[i] are sb_odom_push's outputs.  Each of those per-session pointer arrays may be NULL (that
+ * output is not wanted by any session); an entry may be NULL too.  flags may be NULL (0 for every session).
+ * Rules, checked before any work is enqueued (SB_ERR_INVALID_ARG): all sessions belong to one context, no session
+ * appears twice, no two sessions share a loop-closure detector or a map, all sessions have the same voxel and icp
+ * config (min_points, max_error and the pose may differ), and every session's arguments pass sb_odom_push's checks.
+ * Failure is all or nothing: a call that fails for any session leaves every session, detector and map as it was, and
+ * the message (sb_last_error) names the index of that session.  n == 0 does nothing.  Per call the host waits as often
+ * as one push does, whatever n is. */
+int sb_odom_push_many(sb_odom* const* sessions, int32_t n, const double* const* xyz, const int64_t* n_rows,
+                      const int32_t* frame_idx, const int32_t* flags, sb_odom_frame* out, double* const* out_xyz,
+                      float* const* out_world_f32, double* const* out_desc, sb_loop_result* const* loops,
+                      const int32_t* loop_capacity);
+/* The same for float32 records of stride_floats (>= 3) floats, x, y, z first (sb_odom_push_f32), one stride for all. */
+int sb_odom_push_many_f32(sb_odom* const* sessions, int32_t n, const float* const* xyz, int32_t stride_floats,
+                          const int64_t* n_rows, const int32_t* frame_idx, const int32_t* flags, sb_odom_frame* out,
+                          double* const* out_xyz, float* const* out_world_f32, double* const* out_desc,
+                          sb_loop_result* const* loops, const int32_t* loop_capacity);
+
 /* ---------------------------------------------------------------- multi-GPU exchanges (SURVEY.md 8e) -------- */
 /* One process per GPU; the caller owns the NCCL communicator (an ncclComm_t passed as void*; NCCL itself is looked up
  * in the already-loaded libnccl.so.2 at first use, it is not a link dependency of this library).  The reference has no

@@ -570,6 +570,7 @@ void sb_ctx_destroy(sb_ctx* ctx) {
     cudaFree(c->d_flags);
     for (int i = 0; i < c->ev_created; ++i) cudaEventDestroy(c->ev[i]);
     if (c->pinned) cudaFreeHost(c->pinned);
+    if (c->h_many) cudaFreeHost(c->h_many);
     if (c->h_icp_res) cudaFreeHost(c->h_icp_res);
     if (c->h_icp_passes) cudaFreeHost(c->h_icp_passes);
     if (c->icp_stream) cudaStreamDestroy(c->icp_stream);

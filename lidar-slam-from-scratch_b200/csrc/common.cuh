@@ -103,6 +103,8 @@ struct Ctx {
     unsigned knn_attr_done = 0;    // forest.cu: k_self_knn instantiations whose shared-memory limit has been raised
     i64 last_icp_iterations = 0;   // max history length of the last icp_batch (launches of k_icp_iter)
     i64 last_counts[4] = {0, 0, 0, 0};  // raw rows, downsampled rows, target rows, sum over pairs of n_src * passes
+    char* h_many = nullptr;        // odom_many.cu: pinned staging of the rows of a call, then of its outputs
+    size_t h_many_cap = 0;
 };
 
 // stage ids for stage_mark / sb_ctx_stage_ms

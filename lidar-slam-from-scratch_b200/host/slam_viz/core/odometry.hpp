@@ -5,6 +5,7 @@
 // session.
 #pragma once
 #include <memory>
+#include <stdexcept>
 #include <vector>
 
 #include "icp.hpp"
@@ -81,6 +82,56 @@ public:
         check(sb_odom_push(odom_.get(), scan.points().data(), n, frame_idx, flags, &f, cloud.data(), world.data(), nullptr,
                            raw.data(), max_loops_),
               "Odometry::push");
+        return frame_of(f, cloud, world, raw);
+    }
+
+    // One scan into each of many sessions in one call (sb_odom_push_many): one voxel grid, one index build and one ICP
+    // batch for all of them, with the results of sessions[i]->push(scans[i], frame_idx[i], ...) in order, bit for bit.
+    // The sessions must be distinct, share no detector or map, and have the same voxel size and ICP config.
+    static std::vector<OdometryFrame> push_many(const std::vector<Odometry*>& sessions, const std::vector<PointCloud>& scans,
+                                                const std::vector<int>& frame_idx, bool add_frame = true,
+                                                bool detect = false, bool add_map = true) {
+        const size_t n = sessions.size();
+        if (scans.size() != n || frame_idx.size() != n)
+            throw std::invalid_argument("Odometry::push_many: one scan and one frame index per session");
+        std::vector<sb_odom*> h(n);
+        std::vector<const double*> xyz(n);
+        std::vector<int64_t> rows(n);
+        std::vector<int32_t> idx(n), flags(n), caps(n, max_loops_);
+        std::vector<PointCloud::Matrix> clouds;
+        std::vector<std::vector<float>> worlds(n);
+        std::vector<std::vector<sb_loop_result>> raw(n, std::vector<sb_loop_result>((size_t)max_loops_));
+        std::vector<double*> cloud_p(n);
+        std::vector<float*> world_p(n);
+        std::vector<sb_loop_result*> loop_p(n);
+        clouds.reserve(n);
+        for (size_t i = 0; i < n; ++i) {
+            const Odometry* o = sessions[i];
+            h[i] = o->odom_.get();
+            xyz[i] = scans[i].points().data();
+            rows[i] = (int64_t)scans[i].size();
+            idx[i] = frame_idx[i];
+            flags[i] = (add_frame && o->loop_ ? SB_ODOM_ADD_FRAME : 0) | (detect ? SB_ODOM_DETECT : 0) |
+                       (add_map && o->map_ ? SB_ODOM_ADD_MAP : 0);
+            clouds.emplace_back(rows[i], 3);
+            worlds[i].resize((size_t)(3 * (rows[i] > 0 ? rows[i] : 1)));
+            cloud_p[i] = clouds[i].data();
+            world_p[i] = worlds[i].data();
+            loop_p[i] = raw[i].data();
+        }
+        std::vector<sb_odom_frame> f(n);
+        check(sb_odom_push_many(h.data(), (int32_t)n, xyz.data(), rows.data(), idx.data(), flags.data(), f.data(),
+                                cloud_p.data(), world_p.data(), nullptr, loop_p.data(), caps.data()),
+              "Odometry::push_many");
+        std::vector<OdometryFrame> out;
+        out.reserve(n);
+        for (size_t i = 0; i < n; ++i) out.push_back(frame_of(f[i], clouds[i], worlds[i], raw[i]));
+        return out;
+    }
+
+private:
+    static OdometryFrame frame_of(const sb_odom_frame& f, const PointCloud::Matrix& cloud, const std::vector<float>& world,
+                                  const std::vector<sb_loop_result>& raw) {
         OdometryFrame out;
         out.frame_idx = f.frame_idx;
         out.state = (OdometryFrame::State)f.state;
@@ -108,7 +159,6 @@ public:
         return out;
     }
 
-private:
     LoopClosureDetector* loop_;
     Map* map_;
     std::shared_ptr<sb_odom> odom_;

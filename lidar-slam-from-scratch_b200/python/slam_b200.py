@@ -12,6 +12,7 @@ names and argument meaning to Python callers (tests, bench.py) on top of the C A
     LoopClosureDetector(cfg).addFrame/detect   loop_closure.hpp:41-149
     LoopClosureDetector.addFrames/detect_batch the same over a whole recorded sequence (slam_node.cpp:159-167)
     Odometry(engine).push(scan, i)             SlamNode::process_frame one scan per call (slam_node.cpp:118-175)
+    push_many(sessions, scans, frame_idx)      one scan into each of many sessions in one call (many streams, one GPU)
     Map(engine).add / set_poses / ...          the node's keyframe clouds, poses and occupancy grid on the device
 
 There is no CPU implementation here: if the shared library is missing, or no sm_100 device is usable, construction
@@ -169,6 +170,9 @@ SYMBOLS = {
     "sb_map_global": (C.c_int, [_P, C.c_double, _D, _I64]),
     "sb_map_global_f32": (C.c_int, [_P, C.c_double, C.POINTER(C.c_float), _I64]),
     "sb_odom_create2": (C.c_int, [_P, C.POINTER(OdomConfigC), _P, _P, C.POINTER(_P)]),
+    "sb_odom_push_many": (C.c_int, [_P, C.c_int32, _P, _I64, _I32, _I32, C.POINTER(OdomFrameC), _P, _P, _P, _P, _I32]),
+    "sb_odom_push_many_f32": (C.c_int, [_P, C.c_int32, _P, C.c_int32, _I64, _I32, _I32, C.POINTER(OdomFrameC), _P, _P, _P,
+                                        _P, _I32]),
     "sb_gather_results": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(ICPResultC), C.c_int32, C.POINTER(ICPResultC)]),
     "sb_gather_candidates": (C.c_int, [_P, _P, C.c_int32, _D, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
     "sb_odometry_factors": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_int32, C.c_double, C.POINTER(PoseFactorC)]),
@@ -870,6 +874,72 @@ class Odometry:
         out_desc = desc if (want_desc and state != ODOM_SKIPPED) else None
         res = [LoopClosureDetector._result(loops[i]) for i in range(min(int(fr.n_loops), cap))]
         return OdomFrame(fr, res, out_cloud, out_world, out_desc)
+
+
+def push_many(sessions, frames, frame_idx, add_frame=True, detect=False, add_map=True, want_cloud=False,
+              want_world_f32=False, want_desc=False, loop_capacity=None):
+    """One frame into each of many Odometry sessions of one engine in one call (sb_odom_push_many): one voxel grid, one
+    index build and one ICP batch for all of them.  The results are those of sessions[i].push(frames[i], frame_idx[i],
+    ...) for i in order, bit for bit, and the sessions are left as those pushes would leave them.  frames: (n, 3)
+    float64 rows each, or float32 records of one width for all (n, 3) / (n, 4).  frame_idx, add_frame, detect, add_map
+    and loop_capacity (accepted loops returned per session; default: its detector's max_candidates) may be scalars or one
+    value per session.  Rules (SlamB200Error SB_ERR_INVALID_ARG otherwise): no session twice, no shared detector or map,
+    one voxel and icp config for all.  A call that fails changes no session.  Returns a list of OdomFrame."""
+    n = len(sessions)
+    if len(frames) != n:
+        raise ValueError("one frame per session")
+    if n == 0:
+        return []
+    e = sessions[0].e
+
+    def per(v, name):
+        v = list(v) if isinstance(v, (list, tuple, np.ndarray)) else [v] * n
+        if len(v) != n:
+            raise ValueError(f"{name}: one value per session")
+        return v
+
+    idx, af, dt, am = per(frame_idx, "frame_idx"), per(add_frame, "add_frame"), per(detect, "detect"), per(add_map, "add_map")
+    f32 = isinstance(frames[0], np.ndarray) and frames[0].dtype == np.float32
+    if f32:
+        pts = [np.ascontiguousarray(p) for p in frames]
+        if any(p.dtype != np.float32 or p.ndim != 2 or p.shape[1] != pts[0].shape[1] for p in pts):
+            raise ValueError("float32 frames must all be (n, 3) or all (n, 4) records")
+    else:
+        pts = [_f64(p, 3) for p in frames]
+    rows = np.array([p.shape[0] for p in pts], dtype=np.int64)
+    flags = np.array([(ODOM_ADD_FRAME if af[i] and s.loop is not None else 0) | (ODOM_DETECT if dt[i] else 0) |
+                      (ODOM_ADD_MAP if am[i] and s.map is not None else 0) for i, s in enumerate(sessions)], dtype=np.int32)
+    fi = np.array([int(x) for x in idx], dtype=np.int32)
+    caps = per(loop_capacity, "loop_capacity") if loop_capacity is not None else [
+        max(int(s.loop.cfg.max_candidates), 0) if (dt[i] and s.loop is not None) else 0 for i, s in enumerate(sessions)]
+    cap = np.array([int(c) for c in caps], dtype=np.int32)
+    loops = [(LoopResultC * max(int(c), 1))() for c in cap]
+    clouds = [np.empty((max(int(r), 1), 3)) for r in rows] if want_cloud else None
+    worlds = [np.empty((max(int(r), 1), 3), dtype=np.float32) for r in rows] if want_world_f32 else None
+    descs = [np.empty(SB_SC_SIZE) for _ in range(n)] if want_desc else None
+
+    def ptrs(arrs):
+        return (_P * n)(*[a.ctypes.data for a in arrs]) if arrs is not None else None
+
+    hs = (_P * n)(*[s.h for s in sessions])
+    out = (OdomFrameC * n)()
+    tail = (fi.ctypes.data_as(_I32), flags.ctypes.data_as(_I32), out, ptrs(clouds), ptrs(worlds), ptrs(descs),
+            (_P * n)(*[C.addressof(l) for l in loops]), cap.ctypes.data_as(_I32))
+    xs = ptrs(pts)
+    if f32:
+        st = e.lib.sb_odom_push_many_f32(hs, n, xs, int(pts[0].shape[1]), rows.ctypes.data_as(_I64), *tail)
+    else:
+        st = e.lib.sb_odom_push_many(hs, n, xs, rows.ctypes.data_as(_I64), *tail)
+    e._check(st)
+    res = []
+    for i in range(n):
+        f = out[i]
+        m, state = int(f.n_points), int(f.state)
+        lp = [LoopClosureDetector._result(loops[i][j]) for j in range(min(int(f.n_loops), int(cap[i])))]
+        res.append(OdomFrame(f, lp, clouds[i][:m].copy() if want_cloud else None,
+                             worlds[i][:m].copy() if (want_world_f32 and state != ODOM_SKIPPED) else None,
+                             descs[i] if (want_desc and state != ODOM_SKIPPED) else None))
+    return res
 
 
 class Map:
