@@ -244,6 +244,27 @@ int sb_loop_candidates_batch(sb_loop* loop, const int32_t* query_entries, int32_
 int sb_loop_detect_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_queries,
                          sb_loop_result* results, int32_t* count);
 
+/* Loop closures between detectors: robots of a fleet mapping the same place, or a restarted robot relocalizing against
+ * the database of an earlier run.  dbs[0..n_dbs) are detectors on one context, each at most once, all world == 1 and
+ * with one loop config (every field but frame_gap equal).  Query i is entry query_entry[i] (0-based, as
+ * sb_loop_detect_batch counts) of dbs[query_db[i]]; it gets detect()'s rule (loop_closure.hpp:66-126) over the entries
+ * of every OTHER detector: candidates are the entries with distance < sc_distance_threshold (frame indices of different
+ * streams are unrelated, so there is no frame gap), ordered by (distance, db, entry), and the walk verifies them with
+ * the loop ICP from identity (loop_closure.hpp:99-109), accepts converged ones with final_error < icp_fitness_threshold
+ * and stops at max_candidates acceptances without skipping a candidate.  The query's own detector is never searched.
+ * Queries may come in any order and repeat; neither call modifies a detector; n_queries == 0 does nothing.  A rule
+ * broken returns SB_ERR_INVALID_ARG before any work, with a message naming the detector or query index.
+ *
+ * Stage 1: per query the best min(k, count[i]) candidates over the other detectors, ascending (distance, db, entry):
+ * dist / db / entry [i*k ...]; count[i] = how many are under the threshold.  1 <= k <= SB_LOOP_SELECT_MAX. */
+int sb_loop_candidates_across(sb_loop* const* dbs, int32_t n_dbs, const int32_t* query_db, const int32_t* query_entry,
+                              int32_t n_queries, int32_t k, double* dist, int32_t* db, int32_t* entry, int32_t* count);
+/* detect() across detectors: results / match_db [i*max_candidates ...] hold the count[i] accepted loops of query i
+ * (query_frame = frame of the query entry, match_frame = frame of the matched entry in dbs[match_db]).
+ * max_candidates <= 0 gives empty results (results and match_db may then be NULL). */
+int sb_loop_detect_across(sb_loop* const* dbs, int32_t n_dbs, const int32_t* query_db, const int32_t* query_entry,
+                          int32_t n_queries, sb_loop_result* results, int32_t* match_db, int32_t* count);
+
 /* ---------------------------------------------------------------- streaming odometry session --------------- */
 /* SlamNode::process_frame (slam_node.cpp:118-175) one scan per call, with the previous frame kept on the device: its
  * downsampled cloud, index and normals serve as the next frame's ICP target, so no frame is uploaded or indexed twice.

@@ -1175,6 +1175,82 @@ int sb_loop_detect_batch(sb_loop* loop, const int32_t* query_entries, int32_t n_
     return loop_detect_batch(loop, query_entries, n_queries, results, count);
 }
 
+// rules of the cross-detector calls; the message names the offending detector or query index
+static int check_across(sb_loop* const* dbs, int32_t n_dbs, const int32_t* qdb, const int32_t* qe, int32_t n_q,
+                        std::vector<sb_loop*>& out) {
+    Ctx* c = dbs[0]->ctx;
+    const sb_loop_config& a = dbs[0]->cfg;
+    for (int d = 0; d < n_dbs; ++d) {
+        const sb_loop* L = dbs[d];
+        if (L->ctx != c) return fail(c, SB_ERR_INVALID_ARG, "detector %d is on another context than detector 0", d);
+        for (int o = 0; o < d; ++o)
+            if (dbs[o] == L) return fail(c, SB_ERR_INVALID_ARG, "detector %d appears twice (also detector %d)", d, o);
+        if (L->world != 1) return fail(c, SB_ERR_INVALID_ARG, "detector %d has world %d; search across detectors needs world == 1", d, L->world);
+        const sb_loop_config& b = L->cfg;
+        const char* diff = b.sc_distance_threshold != a.sc_distance_threshold ? "sc_distance_threshold"
+                         : b.icp_fitness_threshold != a.icp_fitness_threshold ? "icp_fitness_threshold"
+                         : b.max_candidates != a.max_candidates ? "max_candidates"
+                         : b.icp_max_iterations != a.icp_max_iterations ? "icp_max_iterations"
+                         : b.normals_k != a.normals_k ? "normals_k"
+                         : b.icp_tolerance != a.icp_tolerance ? "icp_tolerance"
+                         : b.verify_chunk != a.verify_chunk ? "verify_chunk" : nullptr;
+        if (diff) return fail(c, SB_ERR_INVALID_ARG, "detector %d: %s differs from detector 0's", d, diff);
+    }
+    for (int i = 0; i < n_q; ++i) {
+        if (qdb[i] < 0 || qdb[i] >= n_dbs)
+            return fail(c, SB_ERR_INVALID_ARG, "query %d: detector %d out of range [0, %d)", i, qdb[i], n_dbs);
+        const int n = dbs[qdb[i]]->n_global;
+        if (qe[i] < 0 || qe[i] >= n)
+            return fail(c, SB_ERR_INVALID_ARG, "query %d: entry %d out of range [0, %d) of detector %d", i, qe[i], n, qdb[i]);
+    }
+    out.assign(dbs, dbs + n_dbs);
+    return SB_OK;
+}
+
+static bool null_db(sb_loop* const* dbs, int32_t n_dbs) {
+    if (!dbs) return true;
+    for (int d = 0; d < n_dbs; ++d)
+        if (!dbs[d]) return true;
+    return false;
+}
+
+int sb_loop_candidates_across(sb_loop* const* dbs, int32_t n_dbs, const int32_t* query_db, const int32_t* query_entry,
+                              int32_t n_queries, int32_t k, double* dist, int32_t* db, int32_t* entry, int32_t* count) {
+    if (n_dbs < 0 || n_queries < 0 || k < 1 || k > SB_LOOP_SELECT_MAX) return SB_ERR_INVALID_ARG;
+    if (n_queries == 0) return SB_OK;
+    if (n_dbs == 0 || null_db(dbs, n_dbs) || !query_db || !query_entry || !dist || !db || !entry || !count)
+        return SB_ERR_INVALID_ARG;
+    Enter g(dbs[0]->ctx);
+    std::vector<sb_loop*> L;
+    SB_TRY(check_across(dbs, n_dbs, query_db, query_entry, n_queries, L));
+    std::vector<std::vector<std::pair<double, int>>> cand;
+    std::vector<int> total;
+    SB_TRY(loop_candidates_across(L, query_db, query_entry, n_queries, cand, total));
+    std::vector<ScDbRow> tab;
+    loop_across_table(L, tab);
+    for (int i = 0; i < n_queries; ++i) {
+        count[i] = total[i];
+        for (int j = 0; j < k && j < (int)cand[i].size(); ++j) {
+            const size_t o = (size_t)i * k + j;
+            dist[o] = cand[i][j].first;
+            loop_across_decode(tab, cand[i][j].second, &db[o], &entry[o]);
+        }
+    }
+    return SB_OK;
+}
+
+int sb_loop_detect_across(sb_loop* const* dbs, int32_t n_dbs, const int32_t* query_db, const int32_t* query_entry,
+                          int32_t n_queries, sb_loop_result* results, int32_t* match_db, int32_t* count) {
+    if (n_dbs < 0 || n_queries < 0) return SB_ERR_INVALID_ARG;
+    if (n_queries == 0) return SB_OK;
+    if (n_dbs == 0 || null_db(dbs, n_dbs) || !query_db || !query_entry || !count) return SB_ERR_INVALID_ARG;
+    if (dbs[0]->cfg.max_candidates > 0 && (!results || !match_db)) return SB_ERR_INVALID_ARG;
+    Enter g(dbs[0]->ctx);
+    std::vector<sb_loop*> L;
+    SB_TRY(check_across(dbs, n_dbs, query_db, query_entry, n_queries, L));
+    return loop_detect_across(L, query_db, query_entry, n_queries, results, match_db, count);
+}
+
 // ---------------------------------------------------------------- after the path: world frame, map
 void sb_default_grid_config(sb_grid_config* cfg) {  // slam_node.hpp:35-40
     cfg->resolution = 0.2;

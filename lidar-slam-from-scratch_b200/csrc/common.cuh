@@ -428,6 +428,21 @@ int sc_sq_dev(Ctx* ctx, const double* d_desc, int n, double* d_sq);
 // e < n_e of every tile that holds a pair with e < qslot[r] and a frame gap >= frame_gap (d_meta: (frame, entry))
 int sc_distance_many_dev(Ctx* ctx, const double* d_desc, const double* d_sq, const int2* d_meta, const int* d_qslot,
                          int n_q, int n_e, int frame_gap, double* d_dist, i64 ld);
+// Many detectors' pools searched in place: one row per detector, its entries at columns [base, base + count) of a
+// column space in which every detector is padded to a multiple of 8 columns (ld in all).
+struct ScDbRow {
+    const double* desc;   // the detector's descriptor pool
+    int count;            // entries
+    int base;             // first column
+};
+// col_db[c] = detector of column c (-1: padding) and its sums sq[c * 60 ...]; query r (entry qe[r] of detector qdb[r])
+// is gathered to qdesc[r * 1200 ...] with sums at sq[(ld + r) * 60 ...].  One launch.
+int sc_sq_across_dev(Ctx* ctx, const ScDbRow* d_tab, int n_dbs, int ld, const int* d_qdb, const int* d_qe, int n_q,
+                     int* d_col_db, double* d_sq, double* d_qdesc);
+// dist[r * ld + c] for query r of a group (descriptors d_qdesc, sums d_qsq, detectors d_qdb) and every column c of a
+// detector other than d_qdb[r]; tiles whose 64 pairs all belong to the query's own detector are skipped.
+int sc_distance_across_dev(Ctx* ctx, const ScDbRow* d_tab, const int* d_col_db, const double* d_qdesc,
+                           const double* d_qsq, const int* d_qdb, int n_q, const double* d_sq, double* d_dist, i64 ld);
 
 // icp.cu
 int solve_point_to_plane_dev(Ctx* ctx, const double* d_src, const double* d_tgt, const double* d_nrm, i64 n,
@@ -485,6 +500,15 @@ int loop_add_many(sb_loop* L, const double* xyz, const i64* offsets, int n_frame
 int loop_candidates_batch(sb_loop* L, const int* qslots, int n_q, std::vector<std::vector<std::pair<double, int>>>& cand,
                           std::vector<int>& total);
 int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* results, int* count);
+// Across detectors (world == 1, one context, one loop config; checked by the caller): query i is entry qe[i] of
+// dbs[qdb[i]], searched against every entry of every other detector.  Candidate ids are columns of the padded column
+// space loop_across_table lays out (it returns ld, the number of columns); loop_across_decode maps one back.
+int loop_across_table(const std::vector<sb_loop*>& dbs, std::vector<ScDbRow>& tab);
+void loop_across_decode(const std::vector<ScDbRow>& tab, int col, int* db, int* entry);
+int loop_candidates_across(const std::vector<sb_loop*>& dbs, const int* qdb, const int* qe, int n_q,
+                           std::vector<std::vector<std::pair<double, int>>>& cand, std::vector<int>& total);
+int loop_detect_across(const std::vector<sb_loop*>& dbs, const int* qdb, const int* qe, int n_q, sb_loop_result* results,
+                       int* match_db, int* count);
 // loop_add for a cloud and descriptor already in device memory, in two steps: loop_add_enqueue grows the pools and
 // enqueues the device-to-device copies without waiting; loop_add_commit records the entry on the host once the stream
 // has run them.  Together they leave the state loop_add(cloud, frame_idx, desc) leaves; without the commit the

@@ -10,6 +10,8 @@
 #include "common.cuh"
 
 #include <algorithm>
+#include <functional>
+#include <map>
 
 namespace sb {
 
@@ -157,12 +159,24 @@ struct SelList {   // lane j of a warp holds the j-th best pair
     }
 };
 
-// One row: the entries [0, n_db) against a query of frame query_frame.  Shared by the single-query launch and the
-// one-CTA-per-query batch launch (k_loop_select_many), so both select with the same code.
-__device__ __forceinline__ void loop_select_row(const double* __restrict__ dist, const int2* __restrict__ meta, int n_db,
-                                                int query_frame, int frame_gap, double threshold,
-                                                unsigned long long* __restrict__ out_d, int* __restrict__ out_e,
-                                                int* __restrict__ out_total) {
+// Which entries of a row a query may match: keep(i, id) says whether entry i passes and sets the id it is ordered and
+// reported by.  detect() of one detector: the frame gap (loop_closure.hpp:79-81), id = entry.
+struct GapFilter {
+    const int2* __restrict__ meta;
+    int query_frame, frame_gap;
+    __device__ __forceinline__ bool operator()(int i, int& id) const {
+        const int2 mt = meta[i];
+        id = mt.y;
+        return query_frame - mt.x >= frame_gap;
+    }
+};
+
+// One row: the entries [0, n_db) that pass `keep`.  Shared by the single-query launch, the one-CTA-per-query batch
+// launch (k_loop_select_many) and the cross-detector launch (k_loop_select_across), so all select with the same code.
+template <class Keep>
+__device__ __forceinline__ void loop_select_row(const double* __restrict__ dist, int n_db, const Keep& keep,
+                                                double threshold, unsigned long long* __restrict__ out_d,
+                                                int* __restrict__ out_e, int* __restrict__ out_total) {
     __shared__ unsigned long long s_d[32][KSEL];
     __shared__ int s_e[32][KSEL];
     __shared__ int s_total;
@@ -178,14 +192,14 @@ __device__ __forceinline__ void loop_select_row(const double* __restrict__ dist,
         int ce = 0x7fffffff;
         bool ok = false;
         if (i < n_db) {
-            const int2 mt = meta[i];
+            int id;
             const double dv = dist[i];
-            ok = (query_frame - mt.x >= frame_gap) && (dv < threshold);   // loop_closure.hpp:79-81, 86-88 (NaN: false)
+            ok = keep(i, id) && (dv < threshold);   // loop_closure.hpp:79-81, 86-88 (NaN: false)
             if (ok) {   // order-preserving image of the double (a cosine distance can round to -1e-16)
                 const unsigned long long b = (unsigned long long)__double_as_longlong(dv);
                 cd = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
                 if (cd == ~0ull) cd = ~0ull - 1ull;
-                ce = mt.y;
+                ce = id;
                 ++mine;
             }
         }
@@ -220,7 +234,7 @@ __global__ void __launch_bounds__(1024) k_loop_select(const double* __restrict__
                                                       int n_db, int last_frame, int frame_gap, double threshold,
                                                       unsigned long long* __restrict__ out_d, int* __restrict__ out_e,
                                                       int* __restrict__ out_total) {
-    loop_select_row(dist, meta, n_db, last_frame, frame_gap, threshold, out_d, out_e, out_total);
+    loop_select_row(dist, n_db, GapFilter{meta, last_frame, frame_gap}, threshold, out_d, out_e, out_total);
 }
 
 // row r: query slot qslot[r] against the entries below it, distances at dist + r * ld (k_sc_distance_many)
@@ -230,7 +244,29 @@ __global__ void __launch_bounds__(1024) k_loop_select_many(const double* __restr
                                                            unsigned long long* __restrict__ out_d,
                                                            int* __restrict__ out_e, int* __restrict__ out_total) {
     const int r = blockIdx.x, q = qslot[r];
-    loop_select_row(dist + (i64)r * ld, meta, q, meta[q].x, frame_gap, threshold, out_d + (i64)r * KSEL,
+    loop_select_row(dist + (i64)r * ld, q, GapFilter{meta, meta[q].x, frame_gap}, threshold, out_d + (i64)r * KSEL,
+                    out_e + (i64)r * KSEL, out_total + r);
+}
+
+// Across detectors: column i passes iff it is an entry (not padding) of a detector other than the query's.  The id is
+// the column, so (distance, id) order is (distance, detector, entry).
+struct OtherDbFilter {
+    const int* __restrict__ col_db;
+    int query_db;
+    __device__ __forceinline__ bool operator()(int i, int& id) const {
+        const int d = col_db[i];
+        id = i;
+        return d >= 0 && d != query_db;
+    }
+};
+
+// row r: query r of the group (detector qdb[r]) against every column, distances at dist + r * ld (k_sc_distance_across)
+__global__ void __launch_bounds__(1024) k_loop_select_across(const double* __restrict__ dist, i64 ld,
+                                                             const int* __restrict__ col_db, const int* __restrict__ qdb,
+                                                             double threshold, unsigned long long* __restrict__ out_d,
+                                                             int* __restrict__ out_e, int* __restrict__ out_total) {
+    const int r = blockIdx.x;
+    loop_select_row(dist + (i64)r * ld, (int)ld, OtherDbFilter{col_db, qdb[r]}, threshold, out_d + (i64)r * KSEL,
                     out_e + (i64)r * KSEL, out_total + r);
 }
 
@@ -345,73 +381,114 @@ static int slot_of(const sb_loop* L, int entry) {
 // ICP batches of loop verification: at most this many pairs per icp_batch call
 static constexpr int VERIFY_BATCH = 4096;
 
-// loop_closure.hpp:99-109 for a set of (query slot, entry) pairs at once.  The forest indexes every distinct entry
-// cloud once (with normals) and every distinct query cloud once (as a source).
-int loop_verify(sb_loop* L, const int* qslots, const int* entries, const double* dist, int n, sb_loop_result* results,
-                int* converged) {
-    Ctx* ctx = L->ctx;
-    if (n <= 0) return SB_OK;
-    const int n_slots = (int)L->entry_id.size();
-    if (n_slots == 0) return fail(ctx, SB_ERR_EMPTY, "loop: empty database");
-    std::vector<int> tgt_slots, src_slots, tgt_of((size_t)n), src_of((size_t)n);
-    std::vector<int> tree_of_slot((size_t)n_slots, -1), src_of_slot((size_t)n_slots, -1);
-    for (int i = 0; i < n; ++i) {
-        const int qs = qslots[i];
-        if (qs < 0 || qs >= n_slots) return fail(ctx, SB_ERR_INVALID_ARG, "loop: query slot %d out of range", qs);
-        const int slot = slot_of(L, entries[i]);
-        if (slot < 0 || slot == qs)
-            return fail(ctx, SB_ERR_INVALID_ARG, "loop: entry %d is not owned by rank %d", entries[i], L->rank);
-        if (tree_of_slot[slot] < 0) {
-            tree_of_slot[slot] = (int)tgt_slots.size();
-            tgt_slots.push_back(slot);
+struct CloudRef {   // a cloud of the loop-closure database: slot `slot` of detector L
+    const sb_loop* L;
+    int slot;
+};
+
+// loop_closure.hpp:99-109 for n (source cloud, target cloud) pairs, each cloud a slot of some detector, with the loop
+// ICP settings of cfg.  The forest indexes every distinct target cloud once (with normals) and every distinct source
+// cloud once (as a source): one forest_append per detector, targets first, in order of first appearance.
+static int verify_pairs(Ctx* ctx, const sb_loop_config& cfg, const CloudRef* src, const CloudRef* tgt, int n,
+                        sb_icp_result* res) {
+    // distinct clouds grouped by detector: trees[k] = (detector, its slots); index[i] = tree of pair i within its group
+    struct Group {
+        const sb_loop* L;
+        std::vector<int> slots;
+    };
+    auto group = [](const CloudRef* refs, int n, std::vector<Group>& groups, std::vector<int>& tree_of) {
+        std::map<std::pair<const sb_loop*, int>, std::pair<int, int>> seen;   // -> (group, index in group)
+        std::map<const sb_loop*, int> group_of;
+        std::vector<std::pair<int, int>> at((size_t)n);
+        for (int i = 0; i < n; ++i) {
+            auto it = seen.find({refs[i].L, refs[i].slot});
+            if (it == seen.end()) {
+                auto g = group_of.find(refs[i].L);
+                if (g == group_of.end()) {
+                    g = group_of.emplace(refs[i].L, (int)groups.size()).first;
+                    groups.push_back({refs[i].L, {}});
+                }
+                std::vector<int>& sl = groups[(size_t)g->second].slots;
+                it = seen.emplace(std::make_pair(refs[i].L, refs[i].slot), std::make_pair(g->second, (int)sl.size())).first;
+                sl.push_back(refs[i].slot);
+            }
+            at[i] = it->second;
         }
-        if (src_of_slot[qs] < 0) {
-            src_of_slot[qs] = (int)src_slots.size();
-            src_slots.push_back(qs);
-        }
-        tgt_of[i] = tree_of_slot[slot];
-        src_of[i] = src_of_slot[qs];
-    }
-    const int n_tgt = (int)tgt_slots.size();
+        std::vector<int> first((size_t)groups.size() + 1, 0);
+        for (size_t g = 0; g < groups.size(); ++g) first[g + 1] = first[g] + (int)groups[g].slots.size();
+        tree_of.resize((size_t)n);
+        for (int i = 0; i < n; ++i) tree_of[i] = first[(size_t)at[i].first] + at[i].second;
+        return first.back();
+    };
+    std::vector<Group> tgt_groups, src_groups;
+    std::vector<int> tgt_of, src_of;
+    const int n_tgt = group(tgt, n, tgt_groups, tgt_of);
+    const int n_src = group(src, n, src_groups, src_of);
     Forest F;
     F.in_arena = true;
-    int s = forest_reserve(ctx, &F, n_tgt + (int)src_slots.size());
-    if (s == SB_OK) s = forest_append(ctx, &F, L->d_clouds, L->cloud_off.data(), tgt_slots.data(), n_tgt);   // candidates
-    if (s == SB_OK) s = forest_normals(ctx, &F, L->cfg.normals_k, nullptr, nullptr);
-    if (s == SB_OK) s = forest_append(ctx, &F, L->d_clouds, L->cloud_off.data(), src_slots.data(), (int)src_slots.size());
-    std::vector<sb_icp_result> res((size_t)n);
+    int s = forest_reserve(ctx, &F, n_tgt + n_src);
+    for (const Group& g : tgt_groups) {   // candidates
+        if (s == SB_OK) s = forest_append(ctx, &F, g.L->d_clouds, g.L->cloud_off.data(), g.slots.data(), (int)g.slots.size());
+        if (s == SB_OK) s = forest_normals(ctx, &F, cfg.normals_k, nullptr, nullptr);
+    }
+    for (const Group& g : src_groups)     // queries
+        if (s == SB_OK) s = forest_append(ctx, &F, g.L->d_clouds, g.L->cloud_off.data(), g.slots.data(), (int)g.slots.size());
     if (s == SB_OK) {
-        sb_icp_config cfg;
-        sb_default_icp_config(&cfg);
-        cfg.max_iterations = L->cfg.icp_max_iterations;  // loop_closure.hpp:106
-        cfg.tolerance = L->cfg.icp_tolerance;            // loop_closure.hpp:107
-        cfg.normals_k = L->cfg.normals_k;
+        sb_icp_config icfg;
+        sb_default_icp_config(&icfg);
+        icfg.max_iterations = cfg.icp_max_iterations;  // loop_closure.hpp:106
+        icfg.tolerance = cfg.icp_tolerance;            // loop_closure.hpp:107
+        icfg.normals_k = cfg.normals_k;
         for (int b = 0; b < n && s == SB_OK; b += VERIFY_BATCH) {
             const int m = std::min(VERIFY_BATCH, n - b);
             std::vector<PairDesc> pairs((size_t)m);
             for (int i = 0; i < m; ++i) {
-                const int qs = qslots[b + i];
+                const CloudRef& q = src[b + i];
                 memset(&pairs[i], 0, sizeof(PairDesc));
                 pairs[i].src_tree = n_tgt + src_of[b + i];   // source = query cloud (loop_closure.hpp:102)
-                pairs[i].n_src = (int)(L->cloud_off[qs + 1] - L->cloud_off[qs]);
+                pairs[i].n_src = (int)(q.L->cloud_off[q.slot + 1] - q.L->cloud_off[q.slot]);
                 pairs[i].tree = tgt_of[b + i];               // target = candidate cloud (loop_closure.hpp:103)
             }
-            s = icp_batch(ctx, &F, pairs, &cfg, res.data() + b);
+            s = icp_batch(ctx, &F, pairs, &icfg, res + b);
         }
     }
     const cudaError_t sync_err = cudaStreamSynchronize(ctx->stream);
     forest_free(&F);
     if (s != SB_OK) return s;
     if (sync_err != cudaSuccess) return fail(ctx, SB_ERR_CUDA, "loop: verification failed on the device: %s", cudaGetErrorString(sync_err));
+    return SB_OK;
+}
+
+static void fill_result(const CloudRef& q, const CloudRef& t, double dist, const sb_icp_result& r, sb_loop_result* R,
+                        int* converged) {
+    R->query_frame = q.L->frame_idx[q.slot];
+    R->match_frame = t.L->frame_idx[t.slot];
+    memcpy(R->transform, r.transformation, sizeof(R->transform));
+    R->scan_context_distance = dist;
+    R->icp_fitness = r.final_error;
+    *converged = r.converged && r.status == SB_OK;
+}
+
+// loop_closure.hpp:99-109 for a set of (query slot, entry) pairs of one detector at once.
+int loop_verify(sb_loop* L, const int* qslots, const int* entries, const double* dist, int n, sb_loop_result* results,
+                int* converged) {
+    Ctx* ctx = L->ctx;
+    if (n <= 0) return SB_OK;
+    const int n_slots = (int)L->entry_id.size();
+    if (n_slots == 0) return fail(ctx, SB_ERR_EMPTY, "loop: empty database");
+    std::vector<CloudRef> src((size_t)n), tgt((size_t)n);
     for (int i = 0; i < n; ++i) {
-        sb_loop_result& R = results[i];
-        R.query_frame = L->frame_idx[qslots[i]];
-        R.match_frame = L->frame_idx[tgt_slots[tgt_of[i]]];
-        memcpy(R.transform, res[i].transformation, sizeof(R.transform));
-        R.scan_context_distance = dist ? dist[i] : 0.0;
-        R.icp_fitness = res[i].final_error;
-        converged[i] = res[i].converged && res[i].status == SB_OK;
+        const int qs = qslots[i];
+        if (qs < 0 || qs >= n_slots) return fail(ctx, SB_ERR_INVALID_ARG, "loop: query slot %d out of range", qs);
+        const int slot = slot_of(L, entries[i]);
+        if (slot < 0 || slot == qs)
+            return fail(ctx, SB_ERR_INVALID_ARG, "loop: entry %d is not owned by rank %d", entries[i], L->rank);
+        src[i] = {L, qs};
+        tgt[i] = {L, slot};
     }
+    std::vector<sb_icp_result> res((size_t)n);
+    SB_TRY(verify_pairs(ctx, L->cfg, src.data(), tgt.data(), n, res.data()));
+    for (int i = 0; i < n; ++i) fill_result(src[i], tgt[i], dist ? dist[i] : 0.0, res[i], &results[i], &converged[i]);
     return SB_OK;
 }
 
@@ -477,19 +554,19 @@ int loop_add_many(sb_loop* L, const double* xyz, const i64* offsets, int n_frame
     return SB_OK;
 }
 
-// detect() for many query slots (world == 1, ascending).  Every round verifies, for each query that still needs
-// acceptances, its next `chunk` candidates; all pairs of a round go through one forest.  Each query's walk then takes
-// its results in (distance, entry) order and advances by the number of candidates verified, so none is skipped.  A
-// query that exhausts its device-selected short list gets its full sorted list and continues where the list ended.
-int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* results, int* count) {
-    Ctx* ctx = L->ctx;
-    const int maxc = L->cfg.max_candidates;
-    for (int i = 0; i < n_q; ++i) count[i] = 0;
-    if (maxc <= 0 || n_q <= 0) return SB_OK;
-    std::vector<std::vector<std::pair<double, int>>> cand;
-    std::vector<int> total;
-    SB_TRY(loop_candidates_batch(L, qslots, n_q, cand, total));
-    int chunk = L->cfg.verify_chunk > 0 ? L->cfg.verify_chunk : maxc;
+// The walk of detect() (loop_closure.hpp:95-122) for many queries at once.  Every round verifies, for each query that
+// still needs acceptances, its next `chunk` candidates; all pairs of a round go through one verify call.  Each query's
+// walk then takes its results in list order and advances by the number of candidates verified, so none is skipped.  A
+// query that exhausts its short list (fewer entries than total[i]) gets its full sorted list from full_list and
+// continues where the short list ended.  The candidate id of every acceptance goes to accepted_id (if not null).
+using Cands = std::vector<std::pair<double, int>>;
+using WalkVerify = std::function<int(const std::vector<int>& query, const std::vector<int>& id,
+                                     const std::vector<double>& dist, sb_loop_result* res, int* conv)>;
+static int detect_walk(Ctx* ctx, const sb_loop_config& cfg, int n_q, std::vector<Cands>& cand, const std::vector<int>& total,
+                       const std::function<int(int, Cands&)>& full_list, const WalkVerify& verify,
+                       sb_loop_result* results, int* accepted_id, int* count) {
+    const int maxc = cfg.max_candidates;
+    int chunk = cfg.verify_chunk > 0 ? cfg.verify_chunk : maxc;
     if (chunk < 1) chunk = 1;
     std::vector<size_t> pos((size_t)n_q, 0);
     std::vector<char> have_all((size_t)n_q);
@@ -502,14 +579,13 @@ int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* re
             if (pos[i] >= cand[i].size()) {
                 if (have_all[i]) continue;
                 arena_reset(ctx);
-                int t = 0;
-                SB_TRY(loop_candidates(L, cand[i], 0, &t, qslots[i]));   // same order, now complete
+                SB_TRY(full_list(i, cand[i]));   // same order, now complete
                 have_all[i] = 1;
                 if (pos[i] >= cand[i].size()) continue;
             }
             const int m = (int)std::min(cand[i].size() - pos[i], (size_t)chunk);
             for (int t = 0; t < m; ++t) {
-                rq.push_back(qslots[i]);
+                rq.push_back(i);
                 re.push_back(cand[i][pos[i] + t].second);
                 rd.push_back(cand[i][pos[i] + t].first);
             }
@@ -521,15 +597,181 @@ int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* re
         std::vector<sb_loop_result> res((size_t)n);
         std::vector<int> conv((size_t)n);
         arena_reset(ctx);
-        SB_TRY(loop_verify(L, rq.data(), re.data(), rd.data(), n, res.data(), conv.data()));
+        SB_TRY(verify(rq, re, rd, res.data(), conv.data()));
         for (size_t k = 0, p = 0; k < owner.size(); p += (size_t)take[k], ++k) {
             const int i = owner[k];
             for (int t = 0; t < take[k] && count[i] < maxc; ++t)
-                if (conv[p + t] && res[p + t].icp_fitness < L->cfg.icp_fitness_threshold)   // loop_closure.hpp:112
+                if (conv[p + t] && res[p + t].icp_fitness < cfg.icp_fitness_threshold) {   // loop_closure.hpp:112
+                    if (accepted_id) accepted_id[(size_t)i * maxc + count[i]] = re[p + t];
                     results[(size_t)i * maxc + count[i]++] = res[p + t];
+                }
             pos[i] += (size_t)take[k];
         }
     }
+    return SB_OK;
+}
+
+// detect() for many query slots (world == 1, ascending).
+int loop_detect_batch(sb_loop* L, const int* qslots, int n_q, sb_loop_result* results, int* count) {
+    Ctx* ctx = L->ctx;
+    for (int i = 0; i < n_q; ++i) count[i] = 0;
+    if (L->cfg.max_candidates <= 0 || n_q <= 0) return SB_OK;
+    std::vector<Cands> cand;
+    std::vector<int> total;
+    SB_TRY(loop_candidates_batch(L, qslots, n_q, cand, total));
+    auto full_list = [&](int i, Cands& c) -> int {
+        int t = 0;
+        return loop_candidates(L, c, 0, &t, qslots[i]);
+    };
+    WalkVerify verify = [&](const std::vector<int>& q, const std::vector<int>& e, const std::vector<double>& d,
+                            sb_loop_result* res, int* conv) -> int {
+        std::vector<int> qs(q.size());
+        for (size_t k = 0; k < q.size(); ++k) qs[k] = qslots[q[k]];
+        return loop_verify(L, qs.data(), e.data(), d.data(), (int)q.size(), res, conv);
+    };
+    return detect_walk(ctx, L->cfg, n_q, cand, total, full_list, verify, results, nullptr, count);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Across detectors (sb_loop_candidates_across / sb_loop_detect_across): query i is entry qe[i] of dbs[qdb[i]], and its
+// candidates are the entries of every other detector under the threshold, ordered by (distance, detector, entry) —
+// detect()'s rule without the frame gap.  Candidate ids are columns of the padded column space of ScDbRow.
+// ---------------------------------------------------------------------------------------------------------------
+int loop_across_table(const std::vector<sb_loop*>& dbs, std::vector<ScDbRow>& tab) {
+    tab.resize(dbs.size());
+    int ld = 0;
+    for (size_t d = 0; d < dbs.size(); ++d) {
+        const int n = (int)dbs[d]->entry_id.size();
+        tab[d] = {dbs[d]->d_desc, n, ld};
+        ld += (n + 7) / 8 * 8;   // whole tiles (SC_TE = 8): a tile never straddles two detectors
+    }
+    return ld;
+}
+
+void loop_across_decode(const std::vector<ScDbRow>& tab, int col, int* db, int* entry) {
+    // the first detector whose padded columns end after col (padded ends never decrease; an empty detector has none)
+    int lo = 0, hi = (int)tab.size() - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (tab[mid].base + (tab[mid].count + 7) / 8 * 8 > col) hi = mid;
+        else lo = mid + 1;
+    }
+    *db = lo;
+    *entry = col - tab[lo].base;
+}
+
+int loop_candidates_across(const std::vector<sb_loop*>& dbs, const int* qdb, const int* qe, int n_q,
+                           std::vector<Cands>& cand, std::vector<int>& total) {
+    Ctx* ctx = dbs[0]->ctx;
+    cand.assign((size_t)n_q, {});
+    total.assign((size_t)n_q, 0);
+    if (n_q <= 0) return SB_OK;
+    std::vector<ScDbRow> tab;
+    const int ld = loop_across_table(dbs, tab);
+    if (ld <= 0) return SB_OK;   // every detector is empty
+    const int n_dbs = (int)dbs.size();
+    const i64 rows = std::max<i64>(8, (i64)(LOOP_DIST_BYTES / (sizeof(double) * (size_t)ld)) / 8 * 8);
+    ScDbRow* d_tab;
+    int *d_q, *d_col_db;
+    double *d_sq, *d_qdesc, *d_dist;
+    char* d_sel;
+    const size_t sel_bytes = (size_t)n_q * (KSEL * 12 + 4);
+    SB_TRY(arena_get(ctx, (size_t)n_dbs, &d_tab));
+    SB_TRY(arena_get(ctx, (size_t)2 * n_q, &d_q));
+    SB_TRY(arena_get(ctx, (size_t)ld, &d_col_db));
+    SB_TRY(arena_get(ctx, (size_t)(ld + n_q) * SB_SC_SECTORS, &d_sq));
+    SB_TRY(arena_get(ctx, (size_t)n_q * SB_SC_SIZE, &d_qdesc));
+    SB_TRY(arena_get(ctx, (size_t)std::min<i64>(rows, n_q) * ld, &d_dist));
+    SB_TRY(arena_get(ctx, sel_bytes, &d_sel));
+    unsigned long long* d_sel_d = reinterpret_cast<unsigned long long*>(d_sel);
+    int* d_sel_e = reinterpret_cast<int*>(d_sel + (size_t)n_q * KSEL * 8);
+    int* d_tot = d_sel_e + (size_t)n_q * KSEL;
+    std::vector<int> q((size_t)2 * n_q);
+    std::copy(qdb, qdb + n_q, q.begin());
+    std::copy(qe, qe + n_q, q.begin() + n_q);
+    SB_TRY(table_upload(ctx, d_tab, tab.data(), sizeof(ScDbRow) * tab.size()));
+    SB_TRY(table_upload(ctx, d_q, q.data(), sizeof(int) * q.size()));
+    const double thr = dbs[0]->cfg.sc_distance_threshold;
+    SB_TRY(sc_sq_across_dev(ctx, d_tab, n_dbs, ld, d_q, d_q + n_q, n_q, d_col_db, d_sq, d_qdesc));
+    for (i64 g0 = 0; g0 < n_q; g0 += rows) {
+        const int ng = (int)std::min<i64>(rows, n_q - g0);
+        SB_TRY(sc_distance_across_dev(ctx, d_tab, d_col_db, d_qdesc + g0 * SB_SC_SIZE, d_sq + (ld + g0) * SB_SC_SECTORS,
+                                      d_q + g0, ng, d_sq, d_dist, ld));
+        SB_LAUNCH(ctx, k_loop_select_across, (unsigned)ng, 1024, 0, d_dist, (i64)ld, d_col_db, d_q + g0, thr,
+                  d_sel_d + g0 * KSEL, d_sel_e + g0 * KSEL, d_tot + g0);
+    }
+    SB_TRY(pinned_reserve(ctx, sel_bytes));
+    SB_CUDA(ctx, cudaMemcpyAsync(ctx->pinned, d_sel, sel_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const unsigned long long* h_d = reinterpret_cast<const unsigned long long*>(ctx->pinned);
+    const int* h_e = reinterpret_cast<const int*>(ctx->pinned + (size_t)n_q * KSEL * 8);
+    for (int r = 0; r < n_q; ++r) {
+        total[r] = h_e[(size_t)n_q * KSEL + r];
+        decode_selection(h_d + (size_t)r * KSEL, h_e + (size_t)r * KSEL, KSEL, cand[r]);
+    }
+    return SB_OK;
+}
+
+// Query i's complete list (distance, column), sorted: the one-query search against each other detector's pool.
+static int across_full_list(const std::vector<sb_loop*>& dbs, const std::vector<ScDbRow>& tab, int qdb, int qe, Cands& cand) {
+    Ctx* ctx = dbs[0]->ctx;
+    cand.clear();
+    int n = 0;
+    for (const ScDbRow& t : tab) n += t.count;
+    if (n == 0) return SB_OK;
+    double* d_out;
+    SB_TRY(arena_get(ctx, (size_t)n, &d_out));
+    const double* q = dbs[qdb]->d_desc + (size_t)qe * SB_SC_SIZE;
+    for (size_t d = 0, off = 0; d < tab.size(); off += (size_t)tab[d].count, ++d)
+        if ((int)d != qdb) SB_TRY(sc_distance_dev(ctx, q, tab[d].desc, tab[d].count, d_out + off));
+    std::vector<double> dist((size_t)n);
+    SB_CUDA(ctx, cudaMemcpyAsync(dist.data(), d_out, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const double thr = dbs[0]->cfg.sc_distance_threshold;
+    for (size_t d = 0, off = 0; d < tab.size(); off += (size_t)tab[d].count, ++d) {
+        if ((int)d == qdb) continue;
+        for (int e = 0; e < tab[d].count; ++e)
+            if (dist[off + e] < thr) cand.push_back({dist[off + e], tab[d].base + e});   // loop_closure.hpp:86-88
+    }
+    std::sort(cand.begin(), cand.end());   // (distance, column) = (distance, detector, entry)
+    return SB_OK;
+}
+
+int loop_detect_across(const std::vector<sb_loop*>& dbs, const int* qdb, const int* qe, int n_q, sb_loop_result* results,
+                       int* match_db, int* count) {
+    Ctx* ctx = dbs[0]->ctx;
+    const sb_loop_config& cfg = dbs[0]->cfg;
+    const int maxc = cfg.max_candidates;
+    for (int i = 0; i < n_q; ++i) count[i] = 0;
+    if (maxc <= 0 || n_q <= 0) return SB_OK;
+    std::vector<Cands> cand;
+    std::vector<int> total;
+    SB_TRY(loop_candidates_across(dbs, qdb, qe, n_q, cand, total));
+    std::vector<ScDbRow> tab;
+    loop_across_table(dbs, tab);
+    auto full_list = [&](int i, Cands& c) -> int { return across_full_list(dbs, tab, qdb[i], qe[i], c); };
+    WalkVerify verify = [&](const std::vector<int>& q, const std::vector<int>& col, const std::vector<double>& d,
+                            sb_loop_result* res, int* conv) -> int {
+        const int n = (int)q.size();
+        std::vector<CloudRef> src((size_t)n), tgt((size_t)n);
+        for (int k = 0; k < n; ++k) {
+            int db, e;
+            loop_across_decode(tab, col[k], &db, &e);
+            src[k] = {dbs[qdb[q[k]]], qe[q[k]]};
+            tgt[k] = {dbs[db], e};
+        }
+        std::vector<sb_icp_result> icp((size_t)n);
+        SB_TRY(verify_pairs(ctx, cfg, src.data(), tgt.data(), n, icp.data()));
+        for (int k = 0; k < n; ++k) fill_result(src[k], tgt[k], d[k], icp[k], &res[k], &conv[k]);
+        return SB_OK;
+    };
+    std::vector<int> cols((size_t)n_q * maxc);
+    SB_TRY(detect_walk(ctx, cfg, n_q, cand, total, full_list, verify, results, cols.data(), count));
+    for (int i = 0; i < n_q; ++i)
+        for (int j = 0; j < count[i]; ++j) {
+            int e;
+            loop_across_decode(tab, cols[(size_t)i * maxc + j], &match_db[(size_t)i * maxc + j], &e);
+        }
     return SB_OK;
 }
 

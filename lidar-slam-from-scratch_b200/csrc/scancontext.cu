@@ -120,19 +120,19 @@ int sc_distance_dev(Ctx* ctx, const double* d_query_desc, const double* d_db, in
 // operands, same order, separately rounded), so the batch kernel below needs only sum_ab and its distances are the
 // same bits.
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(64) k_sc_sq(const double* __restrict__ desc, double* __restrict__ sq) {
-    __shared__ double sb_[CELLS];   // ring-major
-    const int e = blockIdx.x, s = threadIdx.x;
-    const double* g = desc + (i64)e * CELLS;
+// sum_bb of descriptor g at the 60 shifts, thread s writing out[s]: the loop of k_sc_distance (64 threads, s_ a
+// CELLS-double ring-major staging area)
+__device__ __forceinline__ void sc_sq_one(const double* __restrict__ g, double* __restrict__ out, double* s_) {
+    const int s = threadIdx.x;
     for (int t = s; t < CELLS; t += 64) {
         int j = t / RINGS, i = t - j * RINGS;
-        sb_[i * SECTORS + j] = g[t];
+        s_[i * SECTORS + j] = g[t];
     }
     __syncthreads();
     if (s >= SECTORS) return;
     double sum_bb = 0.0;
     for (int i = 0; i < RINGS; ++i) {
-        const double* br = sb_ + i * SECTORS;
+        const double* br = s_ + i * SECTORS;
         int jj = s;
 #pragma unroll 4
         for (int j = 0; j < SECTORS; ++j) {
@@ -141,7 +141,13 @@ __global__ void __launch_bounds__(64) k_sc_sq(const double* __restrict__ desc, d
             jj = jj + 1 == SECTORS ? 0 : jj + 1;
         }
     }
-    sq[(i64)e * SECTORS + s] = sum_bb;
+    out[s] = sum_bb;
+}
+
+__global__ void __launch_bounds__(64) k_sc_sq(const double* __restrict__ desc, double* __restrict__ sq) {
+    __shared__ double sb_[CELLS];   // ring-major
+    const int e = blockIdx.x;
+    sc_sq_one(desc + (i64)e * CELLS, sq + (i64)e * SECTORS, sb_);
 }
 
 int sc_sq_dev(Ctx* ctx, const double* d_desc, int n, double* d_sq) {
@@ -160,14 +166,14 @@ static constexpr int SC_TQ = 8, SC_TE = 8, SC_QT = SC_TQ / 2, SC_SG = SECTORS / 
 static constexpr int SC_MANY_THREADS = 2 * SC_TE * SC_SG;   // 240
 static constexpr size_t SC_MANY_SMEM = sizeof(double) * CELLS * (SC_TQ + SC_TE) + sizeof(double) * 64;
 
-// dist[r * ld + e] for query r of the group (slot qslot[r]) and every entry e < qslot[r] whose tile survives: a tile is
-// skipped when none of its (query, entry) pairs is causal (e < q) and passes the frame gap (the same int expression as
-// the selection, k_loop_select); distances of pairs the selection filters out are never read.
-__global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_many(const double* __restrict__ desc,
-                                                                     const double* __restrict__ sq,
-                                                                     const int2* __restrict__ meta,
-                                                                     const int* __restrict__ qslot, int n_q, int frame_gap,
-                                                                     double* __restrict__ dist, i64 ld) {
+// The tile of k_sc_distance_many and k_sc_distance_across, one body so that the distance is one piece of code.  The
+// policy P says which pairs exist: P.query(i) is the key of query i of the group (< 0: none, also for i >= n_q), the
+// tile runs iff some (key, entry e0 + e) pair is P.live, and P.n_e(s_q) entries of the tile are read.  Tile query r is
+// descriptor P.qdesc[key] with sum_aa = P.qsq[key * 60]; tile entry e is descriptor P.edesc[P.entry0(e0) + e], column
+// e0 + e of the distance row, with sum_bb at P.esq[(e0 + e) * 60].  dist[(q0 + r) * ld + e0 + e] receives the minimum
+// over the 60 shifts.
+template <class P>
+__device__ __forceinline__ void sc_tile(const P& pol, double* __restrict__ dist, i64 ld) {
     extern __shared__ double smem[];
     double* sa = smem;                    // [SC_TQ][RINGS][SECTORS]
     double* sb_ = smem + SC_TQ * CELLS;   // [SC_TE][RINGS][SECTORS]
@@ -176,27 +182,26 @@ __global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_many(const d
     __shared__ int s_q[SC_TQ];
     const int q0 = blockIdx.y * SC_TQ, e0 = blockIdx.x * SC_TE;
     const int tid = threadIdx.x;
-    if (tid < SC_TQ) s_q[tid] = q0 + tid < n_q ? qslot[q0 + tid] : -1;
+    if (tid < SC_TQ) s_q[tid] = pol.query(q0 + tid);
     __syncthreads();
     bool live = false;
-    if (tid < SC_TQ * SC_TE) {
-        const int q = s_q[tid / SC_TE], e = e0 + tid % SC_TE;
-        live = q >= 0 && e < q && meta[q].x - meta[e].x >= frame_gap;   // loop_closure.hpp:79-81
-    }
+    if (tid < SC_TQ * SC_TE) live = pol.live(s_q[tid / SC_TE], e0 + tid % SC_TE);
     if (!__syncthreads_or(live)) return;
-    int q_hi = 0;
-#pragma unroll
-    for (int r = 0; r < SC_TQ; ++r) q_hi = max(q_hi, s_q[r]);
-    const int n_e = min(SC_TE, q_hi - e0);   // entries of the tile below the last query (>= 1: the tile is live)
+    const int n_e = pol.n_e(s_q, e0);
+    const double* __restrict__ qdesc = pol.qdesc;
+    const double* __restrict__ qsq = pol.qsq;
+    const double* __restrict__ edesc = pol.edesc;
+    const double* __restrict__ esq = pol.esq;
+    const int e_off = pol.entry0(e0);
     for (int t = tid; t < SC_TQ * CELLS; t += SC_MANY_THREADS) {
         const int r = t / CELLS, c = t - r * CELLS;
         const int j = c / RINGS, i = c - j * RINGS;
-        sa[r * CELLS + i * SECTORS + j] = s_q[r] >= 0 ? desc[(i64)s_q[r] * CELLS + c] : 0.0;
+        sa[r * CELLS + i * SECTORS + j] = s_q[r] >= 0 ? qdesc[(i64)s_q[r] * CELLS + c] : 0.0;
     }
     for (int t = tid; t < SC_TE * CELLS; t += SC_MANY_THREADS) {
         const int r = t / CELLS, c = t - r * CELLS;
         const int j = c / RINGS, i = c - j * RINGS;
-        sb_[r * CELLS + i * SECTORS + j] = r < n_e ? desc[(i64)(e0 + r) * CELLS + c] : 0.0;
+        sb_[r * CELLS + i * SECTORS + j] = r < n_e ? edesc[(i64)(e_off + r) * CELLS + c] : 0.0;
     }
     if (tid < SC_TQ * SC_TE) smin_u[tid] = ~0ull;
     __syncthreads();
@@ -236,11 +241,11 @@ __global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_many(const d
             const int qr = h * SC_QT + r;
             const int q = s_q[qr];
             if (q < 0) continue;
-            const double sum_aa = sq[(i64)q * SECTORS];
+            const double sum_aa = qsq[(i64)q * SECTORS];
             double d = 1.7976931348623157e308;
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                const double sum_bb = sq[(i64)e * SECTORS + g + 15 * k];
+                const double sum_bb = esq[(i64)e * SECTORS + g + 15 * k];
                 double norm = sqrt(sum_aa) * sqrt(sum_bb);                     // scan_context.hpp:137
                 double dk = norm < 1e-10 ? 1.0 : 1.0 - acc[r][k] / norm;       // scan_context.hpp:138-141
                 if (!(dk == dk)) dk = 1.7976931348623157e308;                  // NaN never wins (:96)
@@ -260,6 +265,39 @@ __global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_many(const d
     }
 }
 
+// dist[r * ld + e] for query r of the group (slot qslot[r]) and every entry e < qslot[r] whose tile survives: a tile is
+// skipped when none of its (query, entry) pairs is causal (e < q) and passes the frame gap (the same int expression as
+// the selection, k_loop_select); distances of pairs the selection filters out are never read.
+struct ScManyTile {
+    const double* qdesc;   // = desc: queries and entries are slots of one pool
+    const double* qsq;
+    const double* edesc;
+    const double* esq;
+    const int2* meta;
+    const int* qslot;
+    int n_q, frame_gap;
+    __device__ __forceinline__ int query(int i) const { return i < n_q ? qslot[i] : -1; }
+    __device__ __forceinline__ int entry0(int e0) const { return e0; }   // column = slot
+    __device__ __forceinline__ bool live(int q, int e) const {
+        return q >= 0 && e < q && meta[q].x - meta[e].x >= frame_gap;   // loop_closure.hpp:79-81
+    }
+    __device__ __forceinline__ int n_e(const int* s_q, int e0) const {
+        int q_hi = 0;
+#pragma unroll
+        for (int r = 0; r < SC_TQ; ++r) q_hi = max(q_hi, s_q[r]);
+        return min(SC_TE, q_hi - e0);   // entries of the tile below the last query (>= 1: the tile is live)
+    }
+};
+
+__global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_many(const double* __restrict__ desc,
+                                                                     const double* __restrict__ sq,
+                                                                     const int2* __restrict__ meta,
+                                                                     const int* __restrict__ qslot, int n_q, int frame_gap,
+                                                                     double* __restrict__ dist, i64 ld) {
+    const ScManyTile pol{desc, sq, desc, sq, meta, qslot, n_q, frame_gap};
+    sc_tile(pol, dist, ld);
+}
+
 int sc_distance_many_dev(Ctx* ctx, const double* d_desc, const double* d_sq, const int2* d_meta, const int* d_qslot,
                          int n_q, int n_e, int frame_gap, double* d_dist, i64 ld) {
     if (n_q <= 0 || n_e <= 0) return SB_OK;
@@ -267,6 +305,86 @@ int sc_distance_many_dev(Ctx* ctx, const double* d_desc, const double* d_sq, con
     dim3 grid((unsigned)ceil_div(n_e, SC_TE), (unsigned)ceil_div(n_q, SC_TQ));
     SB_LAUNCH(ctx, k_sc_distance_many, grid, SC_MANY_THREADS, SC_MANY_SMEM, d_desc, d_sq, d_meta, d_qslot, n_q,
               frame_gap, d_dist, ld);
+    return SB_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Queries of some detectors against the entries of the others (sb_loop_candidates_across / sb_loop_detect_across).
+// The column space concatenates the detectors' pools in table order, each padded to whole tiles: column c of detector
+// d is entry c - tab[d].base, for c - base < count.  No pool is copied; the kernels read them through the table.
+// ---------------------------------------------------------------------------------------------------------------
+// Block c < ld: column c, col_db[c] = its detector (-1: padding) and its shifted self sums sq[c * 60 ...].  Block ld + r:
+// query r (entry qe[r] of detector qdb[r]): its descriptor is gathered to qdesc[r] and its sums go to sq[(ld + r) * 60].
+// One launch whatever the number of detectors.
+__global__ void __launch_bounds__(64) k_sc_sq_across(const ScDbRow* __restrict__ tab, int n_dbs, int ld,
+                                                     const int* __restrict__ qdb, const int* __restrict__ qe,
+                                                     int* __restrict__ col_db, double* __restrict__ sq,
+                                                     double* __restrict__ qdesc) {
+    __shared__ double sb_[CELLS];   // ring-major
+    const int c = blockIdx.x;
+    const double* g;
+    if (c < ld) {
+        int lo = 0, hi = n_dbs - 1;   // the first detector whose padded columns end after c (an empty one has none)
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (tab[mid].base + (tab[mid].count + SC_TE - 1) / SC_TE * SC_TE > c) hi = mid;
+            else lo = mid + 1;
+        }
+        const int e = c - tab[lo].base;
+        const bool used = e < tab[lo].count;
+        if (threadIdx.x == 0) col_db[c] = used ? lo : -1;
+        if (!used) return;
+        g = tab[lo].desc + (i64)e * CELLS;
+    } else {
+        const int r = c - ld;
+        g = tab[qdb[r]].desc + (i64)qe[r] * CELLS;
+        for (int t = threadIdx.x; t < CELLS; t += 64) qdesc[(i64)r * CELLS + t] = g[t];
+    }
+    sc_sq_one(g, sq + (i64)c * SECTORS, sb_);
+}
+
+int sc_sq_across_dev(Ctx* ctx, const ScDbRow* d_tab, int n_dbs, int ld, const int* d_qdb, const int* d_qe, int n_q,
+                     int* d_col_db, double* d_sq, double* d_qdesc) {
+    if (ld + n_q <= 0) return SB_OK;
+    SB_LAUNCH(ctx, k_sc_sq_across, (unsigned)(ld + n_q), 64, 0, d_tab, n_dbs, ld, d_qdb, d_qe, d_col_db, d_sq, d_qdesc);
+    return SB_OK;
+}
+
+// A tile covers 8 columns of one detector (the padding keeps tiles from straddling two) and 8 queries; the pair of query
+// r and that detector is live iff r belongs to another detector.
+struct ScAcrossTile {
+    const double* qdesc;   // the group's gathered query descriptors
+    const double* qsq;     // their sums: sq[(ld + g0) * 60 ...]
+    const double* edesc;   // the tile's detector pool
+    const double* esq;     // sums of the column space
+    const int* qdb;        // detector of each query of the group
+    int n_q, tile_db, base, count;
+    __device__ __forceinline__ int query(int i) const { return i < n_q ? i : -1; }
+    __device__ __forceinline__ int entry0(int e0) const { return e0 - base; }
+    __device__ __forceinline__ bool live(int q, int) const { return q >= 0 && qdb[q] != tile_db; }
+    __device__ __forceinline__ int n_e(const int*, int e0) const { return min(SC_TE, count - (e0 - base)); }
+};
+
+__global__ void __launch_bounds__(SC_MANY_THREADS, 1) k_sc_distance_across(const ScDbRow* __restrict__ tab,
+                                                                       const int* __restrict__ col_db,
+                                                                       const double* __restrict__ qdesc,
+                                                                       const double* __restrict__ qsq,
+                                                                       const int* __restrict__ qdb, int n_q,
+                                                                       const double* __restrict__ sq,
+                                                                       double* __restrict__ dist, i64 ld) {
+    const int d = col_db[blockIdx.x * SC_TE];   // a tile's first column is never padding
+    const ScDbRow t = tab[d];
+    const ScAcrossTile pol{qdesc, qsq, t.desc, sq, qdb, n_q, d, t.base, t.count};
+    sc_tile(pol, dist, ld);
+}
+
+int sc_distance_across_dev(Ctx* ctx, const ScDbRow* d_tab, const int* d_col_db, const double* d_qdesc,
+                           const double* d_qsq, const int* d_qdb, int n_q, const double* d_sq, double* d_dist, i64 ld) {
+    if (n_q <= 0 || ld <= 0) return SB_OK;
+    SB_CUDA(ctx, cudaFuncSetAttribute(k_sc_distance_across, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SC_MANY_SMEM));
+    dim3 grid((unsigned)(ld / SC_TE), (unsigned)ceil_div(n_q, SC_TQ));
+    SB_LAUNCH(ctx, k_sc_distance_across, grid, SC_MANY_THREADS, SC_MANY_SMEM, d_tab, d_col_db, d_qdesc, d_qsq, d_qdb, n_q,
+              d_sq, d_dist, ld);
     return SB_OK;
 }
 

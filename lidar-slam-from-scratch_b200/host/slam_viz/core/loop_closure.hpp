@@ -86,8 +86,8 @@ public:
 
     // extension: the underlying detector (b200::Odometry adds frames to it and runs its detect())
     sb_loop* handle() const { return loop_.get(); }
+    const LoopClosureConfig& config() const { return config_; }
 
-private:
     static LoopClosureResult result(const sb_loop_result& raw) {
         LoopClosureResult r;
         r.query_frame = raw.query_frame;
@@ -101,5 +101,36 @@ private:
     LoopClosureConfig config_;
     std::shared_ptr<sb_loop> loop_;
 };
+
+namespace b200 {
+
+struct AcrossLoop {
+    int match_db;          // index in the detector list of the matched entry's detector
+    LoopClosureResult r;   // match_frame: frame of the matched entry; query_frame: frame of the query entry
+};
+
+// extension: loop closures between detectors (sb_loop_detect_across).  queries: (detector index, entry) pairs; each
+// is matched against every entry of every other detector by detect()'s rule without the frame gap.  The detectors
+// share one context and one config.
+inline std::vector<std::vector<AcrossLoop>> detectAcross(const std::vector<LoopClosureDetector*>& dbs,
+                                                         const std::vector<std::pair<int, int>>& queries) {
+    const size_t n = queries.size();
+    std::vector<std::vector<AcrossLoop>> out(n);
+    if (n == 0) return out;
+    const int cap = !dbs.empty() && dbs[0]->config().max_candidates > 0 ? dbs[0]->config().max_candidates : 0;
+    std::vector<sb_loop*> h;
+    for (const LoopClosureDetector* d : dbs) h.push_back(d->handle());
+    std::vector<int32_t> qdb, qe, count(n, 0), mdb(n * (size_t)cap > 0 ? n * (size_t)cap : 1);
+    for (const auto& q : queries) { qdb.push_back(q.first); qe.push_back(q.second); }
+    std::vector<sb_loop_result> raw(mdb.size());
+    check(sb_loop_detect_across(h.data(), (int32_t)h.size(), qdb.data(), qe.data(), (int32_t)n, raw.data(), mdb.data(),
+                                count.data()), "detectAcross");
+    for (size_t i = 0; i < n; ++i)
+        for (int j = 0; j < count[i]; ++j)
+            out[i].push_back({mdb[i * (size_t)cap + j], LoopClosureDetector::result(raw[i * (size_t)cap + j])});
+    return out;
+}
+
+}  // namespace b200
 
 }  // namespace slam

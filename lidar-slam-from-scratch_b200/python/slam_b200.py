@@ -144,6 +144,10 @@ SYMBOLS = {
     "sb_loop_add_frames": (C.c_int, [_P, _D, _I64, C.c_int32, _I32, _D]),
     "sb_loop_candidates_batch": (C.c_int, [_P, _I32, C.c_int32, C.c_int32, _D, _I32, _I32]),
     "sb_loop_detect_batch": (C.c_int, [_P, _I32, C.c_int32, C.POINTER(LoopResultC), _I32]),
+    "sb_loop_candidates_across": (C.c_int, [C.POINTER(_P), C.c_int32, _I32, _I32, C.c_int32, C.c_int32, _D, _I32, _I32,
+                                            _I32]),
+    "sb_loop_detect_across": (C.c_int, [C.POINTER(_P), C.c_int32, _I32, _I32, C.c_int32, C.POINTER(LoopResultC), _I32,
+                                        _I32]),
     "sb_odometry_poses": (C.c_int, [_P, C.POINTER(ICPResultC), C.c_int32, C.c_double, _D, _D]),
     "sb_default_odom_config": (None, [C.POINTER(OdomConfigC)]),
     "sb_odom_create": (C.c_int, [_P, C.POINTER(OdomConfigC), _P, C.POINTER(_P)]),
@@ -766,6 +770,51 @@ class LoopClosureDetector:
         cnt = np.zeros(max(n, 1), dtype=np.int32)
         self.e._check(self.e.lib.sb_loop_detect_batch(self.h, q.ctypes.data_as(_I32), n, res, cnt.ctypes.data_as(_I32)))
         return [[self._result(res[i * m + j]) for j in range(cnt[i])] for i in range(n)]
+
+
+def _across_args(dbs, queries):
+    if len(dbs) == 0:
+        raise ValueError("no detectors")
+    q = np.asarray(queries, dtype=np.int32).reshape(-1, 2) if len(queries) else np.zeros((0, 2), dtype=np.int32)
+    qdb = np.ascontiguousarray(q[:, 0])
+    qe = np.ascontiguousarray(q[:, 1])
+    hs = (_P * len(dbs))(*[d.h for d in dbs])
+    return dbs[0].e, hs, qdb, qe, q.shape[0]
+
+
+def candidates_across(dbs, queries, k=SB_LOOP_SELECT_MAX):
+    """Stage 1 of detect() across detectors (sb_loop_candidates_across).  dbs: LoopClosureDetector objects of one engine
+    (world 1, one loop config); queries: (db_index, entry) pairs.  Query i is searched against every entry of every
+    other detector, without a frame gap.  Returns per query the best min(k, count) candidates as arrays (dist, db,
+    entry), ascending by (distance, db, entry), and the number of candidates under the threshold."""
+    e, hs, qdb, qe, n = _across_args(dbs, queries)
+    dist = np.empty((max(n, 1), k))
+    db = np.empty((max(n, 1), k), dtype=np.int32)
+    ent = np.empty((max(n, 1), k), dtype=np.int32)
+    cnt = np.zeros(max(n, 1), dtype=np.int32)
+    e._check(e.lib.sb_loop_candidates_across(hs, len(dbs), qdb.ctypes.data_as(_I32), qe.ctypes.data_as(_I32), n, int(k),
+                                             _dp(dist), db.ctypes.data_as(_I32), ent.ctypes.data_as(_I32),
+                                             cnt.ctypes.data_as(_I32)))
+    out = []
+    for i in range(n):
+        m = min(int(cnt[i]), k)
+        out.append((dist[i, :m].copy(), db[i, :m].copy(), ent[i, :m].copy()))
+    return out, cnt[:n].copy()
+
+
+def detect_across(dbs, queries):
+    """detect() across detectors (sb_loop_detect_across): per query the list of accepted loops, dicts as
+    LoopClosureDetector.detect returns them plus match_db, the index in dbs of the matched entry's detector
+    (match_frame is that entry's frame, query_frame the query entry's)."""
+    e, hs, qdb, qe, n = _across_args(dbs, queries)
+    m = max(int(dbs[0].cfg.max_candidates), 0)
+    res = (LoopResultC * max(n * m, 1))()
+    mdb = np.zeros(max(n * m, 1), dtype=np.int32)
+    cnt = np.zeros(max(n, 1), dtype=np.int32)
+    e._check(e.lib.sb_loop_detect_across(hs, len(dbs), qdb.ctypes.data_as(_I32), qe.ctypes.data_as(_I32), n, res,
+                                         mdb.ctypes.data_as(_I32), cnt.ctypes.data_as(_I32)))
+    return [[dict(LoopClosureDetector._result(res[i * m + j]), match_db=int(mdb[i * m + j])) for j in range(cnt[i])]
+            for i in range(n)]
 
 
 class OdomFrame:
